@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — beam-8 + RNNLM joint CTC/attention decode throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): char (31-token) VGG+BLSTM CTC-attention model with
 librispeech_asr.yaml dims + random-init 4x1024 RNNLM, beam 8, ctc_weight 0.5, lm_weight 0.5,
@@ -17,7 +17,8 @@ prefix-score step kernel, timed live with CUDA events around every launch; ``pha
 per-phase breakdown of a pass (max over ranks); ``nbest_parity`` compares the run's own N-best of
 the 16 bench-set utterances in tests/golden/beam_nbest_fullsize.npz with the reference's;
 ``sharded_equals_single`` (N > 1) is the bit-for-bit check of the gathered result against rank 0's
-own decode of the last rank's shard.
+own decode of the last rank's shard.  ``--dump-outputs DIR`` writes the N-best arrays of the last timed pass
+(``dump_outputs``); inputs and weights are seeded, so runs with the same arguments decode the same data.
 ``--impl reference`` times the UNMODIFIED reference on the host cores: its decode path byte-compiled
 into oracle/_ref by __graft_entry__.build() (oracle/ref_stage.py), driven through
 bin/test_asr.py::beam_decode and joblib.Parallel on a length-stratified sample of the same set.
@@ -180,6 +181,34 @@ def golden_parity(tok, sc, ln, avg, nn, tie_tol=5e-4, score_tol=2e-4):
     return out
 
 
+DUMP_BYTES = 64 * 1000 * 1000
+
+
+def dump_outputs(out_dir, tok, sc, ln, avg, n, budget=DUMP_BYTES):
+    """Write the N-best arrays of a pass (what ``BeamDecoder.decode_batch(..., return_arrays=True)`` returns, indexed by
+    utterance) to ``out_dir`` as float32 .npy files: ``tokens`` and ``token_scores`` [U, beam, width], ``lengths`` and
+    ``mean_scores`` [U, beam], ``nbest`` [U], plus ``utterance_ids`` (float64) naming each row.  Entries a caller never
+    reads (past a hypothesis' length, hypotheses past the N-best count) are written as 0, so two builds can be compared
+    array for array.  If all rows would take more than ``budget`` bytes, a fixed seeded sample of utterances is written,
+    in id order."""
+    tok, sc, ln, avg, n = (t.cpu().numpy() for t in (tok, sc, ln, avg, n))
+    n_utts, beam, width = tok.shape
+    row_bytes = 4 * (2 * beam * width + 2 * beam + 1) + 8
+    room = budget - 6 * 1024                                      # the six .npy headers
+    ids = np.arange(n_utts)
+    if n_utts * row_bytes > room:
+        ids = np.sort(np.random.default_rng(0).choice(n_utts, room // row_bytes, replace=False))
+    hyp = np.arange(beam)[None, :] < n[ids, None]
+    pos = hyp[:, :, None] & (np.arange(width)[None, None, :] < ln[ids, :, None])
+    arrays = {"tokens": np.where(pos, tok[ids], 0), "token_scores": np.where(pos, sc[ids], 0),
+              "lengths": np.where(hyp, ln[ids], 0), "mean_scores": np.where(hyp, avg[ids], 0), "nbest": n[ids]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+    np.save(os.path.join(out_dir, "utterance_ids.npy"), ids.astype(np.float64))
+    return ids
+
+
 # ------------------------------------------------------------------------------------------------
 # B200 arm
 # ------------------------------------------------------------------------------------------------
@@ -282,6 +311,9 @@ def run_b200(args):
         return float(vals[0].item()), ops.launch_count() - l0, clocks, local_buf, full, phases
 
     ms, launches, clocks, local_buf, full, phases = timed(False, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        # unpacked here: the e2e leg below reads back into the same pinned host buffer
+        dump_outputs(args.dump_outputs, *shard.unpack_nbest_ragged(full, shards, lengths, BEAM, MAX_RATIO, rsize))
     # prefix-score kernel: per-launch CUDA-event durations collected inside the timed region
     ev = dec.prefix_events
     k_ms = [a.elapsed_time(b) for a, b, _, _ in ev]
@@ -612,7 +644,14 @@ def main():
                     "cpu_baseline leg; the reference arm decodes a length-stratified sample of the set unless a length is given)")
     ap.add_argument("--no-as-shipped", action="store_true", help="reference arm: skip the as-shipped (--njobs 4) measurement")
     ap.add_argument("--as-shipped-sample", type=int, default=8, help="reference arm: utterances of the as-shipped measurement")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="B200 arm: write the N-best of the last timed pass to DIR/<name>.npy (float arrays, at most 64 MB; "
+                         "a fixed seeded sample of the utterances when the whole set is larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the B200 arm's outputs")
     args.ragged_h2d = not args.padded_h2d
     if args.impl == "reference":
         run_reference(args)

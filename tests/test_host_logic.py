@@ -231,9 +231,11 @@ def test_memory_budget_splits_a_subword_set_and_keeps_the_char_set_whole():
 
 
 def test_bench_reference_arm_prints_the_contract_line():
-    """`bench.py --impl reference` (the arm the driver times next to ours) on a tiny bounded sample: one JSON line with the
-    contract's keys, no GPU needed, rank != 0 exits silently."""
+    """`bench.py --impl reference` (the CPU arm timed next to the B200 one) on a tiny bounded sample: one JSON line with the
+    result keys, no GPU needed, rank != 0 exits silently.  It times the unmodified reference where that can be imported
+    (oracle/refload.py) and otherwise the oracle port, which it must then name as such."""
     import json, os, subprocess, sys
+    from oracle import refload
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     cmd = [sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
            "--cpu-sample", "2", "--cpu-frames", "40", "--cpu-procs", "2", "--as-shipped-sample", "1"]
@@ -244,13 +246,51 @@ def test_bench_reference_arm_prints_the_contract_line():
     d = json.loads(lines[0])
     assert d["impl"] == "reference" and d["unit"] == "utts/s" and d["higher_is_better"] is True and d["value"] > 0
     assert d["e2e"] == {"value": d["value"], "unit": "utts/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
-    assert d["cpu_baseline"]["kind"] == "reference" and d["cpu_baseline"]["cores"] == 2 and d["gpu_launches"] == 0
+    assert d["cpu_baseline"]["cores"] == 2 and d["gpu_launches"] == 0
     assert "unmodified reference" in d["cpu_baseline"]["sample"] and "quantile" not in d["cpu_baseline"]["sample"]   # fixed-length smoke sample
-    assert d["cpu_baseline"]["as_shipped"]["n_jobs"] == 4 and d["cpu_baseline"]["as_shipped"]["value"] > 0
+    if refload.available() or refload.staged_available():
+        assert d["cpu_baseline"]["kind"] == "reference"
+        assert d["cpu_baseline"]["as_shipped"]["n_jobs"] == 4 and d["cpu_baseline"]["as_shipped"]["value"] > 0
+    else:
+        # the as-shipped leg runs the reference's own settings, so it needs the reference itself
+        assert d["cpu_baseline"]["kind"] == "port" and "oracle port" in d["cpu_baseline"]["sample"]
+        assert d["cpu_baseline"]["as_shipped"] is None
     po = d["cpu_baseline"]["prefix_only"]                          # SURVEY §8d: cheap_compute alone, the kernel-level CPU figure
     assert po["cores"] == 1 and 1e4 < po["cand_frames_per_s"] < 1e9 and "cheap_compute" in po["sample"]
     quiet = subprocess.run(cmd, capture_output=True, text=True, timeout=300, cwd=root, env=dict(os.environ, RANK="1", WORLD_SIZE="2"))
     assert quiet.returncode == 0 and quiet.stdout.strip() == ""
+
+
+def test_bench_dump_outputs_zeroes_unread_entries_and_samples_under_the_budget(tmp_path):
+    """bench.dump_outputs (--dump-outputs): float arrays only, what a caller reads is written as it is and the rest is 0, and
+    over the byte budget a seeded sample of the utterances (the same every time, in id order) keeps the files under it."""
+    import bench
+    g = torch.Generator().manual_seed(0)
+    U, B, W = 50, 3, 7
+    tok = torch.randint(2, 31, (U, B, W), generator=g, dtype=torch.int32)
+    sc = -torch.rand(U, B, W, generator=g)
+    ln = torch.randint(1, W + 1, (U, B), generator=g, dtype=torch.int32)
+    avg = -torch.rand(U, B, generator=g)
+    n = torch.randint(0, B + 1, (U,), generator=g, dtype=torch.int32)
+    names = ["lengths", "mean_scores", "nbest", "token_scores", "tokens", "utterance_ids"]
+    assert bench.dump_outputs(str(tmp_path / "all"), tok, sc, ln, avg, n).tolist() == list(range(U))
+    assert sorted(os.listdir(str(tmp_path / "all"))) == [k + ".npy" for k in names]
+    d = {k: np.load(str(tmp_path / "all" / (k + ".npy"))) for k in names}
+    assert all(a.dtype in (np.float32, np.float64) for a in d.values())
+    assert d["tokens"].shape == d["token_scores"].shape == (U, B, W) and d["nbest"].tolist() == n.tolist()
+    for u in range(U):
+        for k in range(B):
+            m = int(ln[u, k]) if k < int(n[u]) else 0
+            assert d["tokens"][u, k, :m].tolist() == tok[u, k, :m].tolist() and not d["tokens"][u, k, m:].any()
+            assert np.array_equal(d["token_scores"][u, k, :m], sc[u, k, :m].numpy()) and not d["token_scores"][u, k, m:].any()
+            assert d["lengths"][u, k] == m and d["mean_scores"][u, k] == (avg[u, k].item() if k < int(n[u]) else 0.0)
+    budget = 6 * 1024 + 20 * (4 * (2 * B * W + 2 * B + 1) + 8)
+    a = bench.dump_outputs(str(tmp_path / "a"), tok, sc, ln, avg, n, budget=budget)
+    b = bench.dump_outputs(str(tmp_path / "b"), tok, sc, ln, avg, n, budget=budget)
+    assert len(a) == 20 and a.tolist() == b.tolist() == sorted(set(a.tolist()))
+    assert sum(os.path.getsize(str(tmp_path / "a" / f)) for f in os.listdir(str(tmp_path / "a"))) <= budget
+    assert np.load(str(tmp_path / "a" / "utterance_ids.npy")).tolist() == a.tolist()
+    assert np.array_equal(np.load(str(tmp_path / "a" / "tokens.npy")), d["tokens"][a])
 
 
 def test_ragged_nbest_buffer_layout_and_size():
