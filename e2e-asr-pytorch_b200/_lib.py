@@ -61,6 +61,10 @@ SIGNATURES = {
     "e2e_attention_loc_full": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                        c_float, c_float, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                                        c_void_p, c_void_p, c_void_p]),
+    "e2e_attention_loc_heads_supported": (c_int, [c_int, c_int, c_int, c_int, c_int]),
+    "e2e_attention_loc_heads": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                        c_float, c_float, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                                        c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "e2e_lstm_split_rows": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, c_int, c_int, c_void_p, ctypes.c_longlong, c_int, c_int, c_void_p]),
     "e2e_lstm_split_rows_multi": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     "e2e_lstm_cell": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,

@@ -243,6 +243,43 @@ def attention_loc_full(key_t, value, query, prev_att, enc_len, w_conv, w_proj, w
     return attn, ctx
 
 
+def attention_loc_heads_supported(beam, heads, dim, n_filt, width):
+    """Whether e2e_attention_loc_heads launches for this shape (the launcher's own size computation)."""
+    return bool(L.load().e2e_attention_loc_heads_supported(int(beam), int(heads), int(dim), int(n_filt), int(width)))
+
+
+def attention_loc_heads(key_t, value, query, prev_att, enc_len, w_conv, w_proj, w_energy, b_energy, temperature, beam,
+                        per_head_values, n_run=None, hyps_per_unit=0, attn=None, ctx=None):
+    """The multi-head location-aware attention step for the first ``n_run`` utterances: key_t [U,H,A,T] (channel-major
+    keys per head), value [U,T,E] shared by the heads or [U,T,H*E] (``per_head_values``), query [>=n_run*B,H*A],
+    prev_att [>=n_run*B,H,T], w_conv [K,H,W] -> (attn [n_run*B,H,T], ctx [n_run*B,H*E], merge_head's input)."""
+    for t, nm in ((key_t, "key_t"), (value, "value"), (query, "query"), (prev_att, "prev_att"), (w_conv, "w_conv"),
+                  (w_proj, "w_proj"), (w_energy, "w_energy")):
+        _chk(t, F32, nm)
+    _chk(enc_len, I32, "enc_len")
+    u, h, a, t_len = key_t.shape
+    k, h_w, w = w_conv.shape
+    e = value.shape[2] // h if per_head_values else value.shape[2]
+    n_run = u if n_run is None else int(n_run)
+    n = n_run * beam
+    if (h_w != h or value.shape[0] != u or value.shape[1] != t_len or (per_head_values and value.shape[2] != h * e)
+            or prev_att.shape[-1] != t_len or n_run > u):
+        raise ValueError("attention_loc_heads: inconsistent shapes")
+    _chk(query, F32, "query", n * h * a)
+    _chk(prev_att, F32, "prev_att", n * h * t_len)
+    if attn is None:
+        attn = torch.empty((n, h, t_len), dtype=F32, device=key_t.device)
+    if ctx is None:
+        ctx = torch.empty((n, h * e), dtype=F32, device=key_t.device)
+    _chk(attn, F32, "attn", n * h * t_len)
+    _chk(ctx, F32, "ctx", n * h * e)
+    L.check(L.load().e2e_attention_loc_heads(L.ptr(key_t), L.ptr(value), L.ptr(query), L.ptr(prev_att), L.ptr(enc_len),
+                                            L.ptr(w_conv), L.ptr(w_proj), L.ptr(w_energy), float(b_energy), float(temperature),
+                                            n_run, int(beam), int(h), int(t_len), int(a), int(k), int(w), int(e),
+                                            int(bool(per_head_values)), int(hyps_per_unit), L.ptr(attn), L.ptr(ctx), _stream()))
+    return attn, ctx
+
+
 def lstm_split_rows(src, row_idx, n, dst, k, off, scale=None):
     """dst[r, p*k + off : p*k + off + w] = p-th piece of src[row_idx[r]] (src [*,w] fp32).  dst bf16 [>=n, 3k]: the exact
     3-piece split; dst fp16 [>=n, 2k] (``scale`` = a power of two): the 2-piece split of scale*src."""

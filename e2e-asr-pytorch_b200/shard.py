@@ -42,25 +42,31 @@ def plan_shards(lengths, world_size, max_len_ratio=0.2):
 
 
 def estimate_decode_bytes(n_utts, l_max, vocab, beam, n_cand, feat_dim=160, enc_dim=640, att_dim=300,
-                          lm_dim=1024, lm_layers=4, encoder_chunk=128):
+                          lm_dim=1024, lm_layers=4, encoder_chunk=128, num_head=1, v_proj=False):
     """Upper estimate of the HBM ``BeamDecoder.decode_batch`` needs at its peak for ``n_utts`` utterances padded
     to ``l_max`` input frames (DESIGN.md §3: every buffer is sized by the LONGEST utterance of the batch).
     Dominant terms: the frame-major posteriors together with the CTC logits they are made from
     (2 x U x Tmax x Vp fp32 — 170 GB for 2620 utterances with a 10k subword vocabulary), the two prefix-state
-    buffers, the encoder output and the attention keys; the encoder's chunk temporaries are a constant."""
+    buffers, the encoder output and the attention keys; the encoder's chunk temporaries are a constant.  With
+    ``num_head`` heads the keys and alignments are H times as large, and with ``v_proj`` the projected values
+    [U][T][H*enc_dim] are held as well (~22 GB for 2620 utterances of ~828 frames at H = 4), counted twice because the
+    plain multi-head step holds a head-major copy beside them while it makes it."""
     u, t = int(n_utts), (int(l_max) // 4 + 3) // 4 * 4
     vp = (int(vocab) + 3) // 4 * 4
     n = u * beam
     feats = u * int(l_max) * feat_dim * 4
     enc = u * t * enc_dim * 4 * 2                                   # padded output + the packed frames it is scattered from
-    keys = u * t * att_dim * 4 * 2                                  # proj_k output and its channel-major copy
+    h = int(num_head)
+    keys = u * t * att_dim * h * 4 * 2                              # proj_k output and its channel-major copy
+    # tanh(proj_v(enc)) (no projection: the encoder output), twice: the plain multi-head step re-lays it out head-major
+    values = u * t * enc_dim * h * 4 * 2 if v_proj else 0
     post = 2 * u * t * vp * 4 + u * t * 8                           # logits + posteriors (+ blank running sum)
     states = 2 * u * t * beam * max(1, n_cand) * 8
-    attn = 3 * n * t * 4
+    attn = 3 * n * h * t * 4
     lstm = n * (lm_layers * (3 * 2 * lm_dim * 2 + 4 * lm_dim * 4) + 4 * lm_dim * 4) + 3 * n * vp * 4
     hist = 3 * (int(l_max) // 5 + 2) * n * 4
     chunk = min(u, encoder_chunk) * int(l_max) * 40 * 128 * 4 * 3 + (3 << 30) * 2      # VGG activations + unfolded operand + GEMM result
-    return int(1.1 * (feats + enc + keys + post + states + attn + lstm + hist + chunk))
+    return int(1.1 * (feats + enc + keys + values + post + states + attn + lstm + hist + chunk))
 
 
 def make_batches(indices, lengths, max_utts=512, max_padded_frames=None, max_bytes=None, bytes_fn=None):

@@ -29,7 +29,9 @@ PyTorch restatement below runs.  What keeps the step fast without leaving fp32:
 * ``fused_attention``: the location-aware energies + masked softmax run in one
   hand-written kernel (csrc/attention_full.cu: location convolution, energies, masked
   softmax and the context product) instead of a cuDNN convolution, ~8 passes over
-  [U*B, T, 300] temporaries and a batched GEMM, and never touches padded frames;
+  [U*B, T, 300] temporaries and a batched GEMM, and never touches padded frames; multi-head models
+  (attention.num_head = H <= 4) run the same kernel's multi-head form followed by merge_head, and fall back to
+  a plain PyTorch multi-head step for what that kernel's shape query refuses (and for scaled-dot attention);
 * the LSTM states are never permuted: a step reads them through the parents' row index
   (``_FusedLstm``), and the encoder runs over packed frames (``model.Encoder.forward_ragged_packed``).
 """
@@ -336,8 +338,6 @@ class _FusedLstm:
 class BatchedStepper:
     def __init__(self, asr, lm=None, split_gemm=False, fused_attention=False, lm_split="bf16x3", vgg_split="bf16x3", step_graphs=False):
         att = asr.attention
-        if att.num_head != 1:
-            raise NotImplementedError("multi-head attention is not supported by the batched beam search")
         if att.mode not in ("loc", "dot"):
             raise NotImplementedError("attention mode " + str(att.mode))
         self.asr, self.lm = asr, lm
@@ -346,6 +346,7 @@ class BatchedStepper:
             raise ValueError("unknown split format " + str(vgg_split))
         self.vgg_split = vgg_split               # their operand format
         self.mode, self.temperature = att.mode, att.att_layer.temperature
+        self.H = att.num_head
         # fused device LSTM steps (csrc/lstm_step.cu) whenever the weights live on a GPU; the plain
         # PyTorch cells otherwise (CPU tests of the host logic, GRU models)
         def make(rnn, table=None, split="bf16x3"):
@@ -359,12 +360,15 @@ class BatchedStepper:
             if isinstance(stack, _FusedLstm):
                 stack.use_graphs = bool(step_graphs)
         self.mark = lambda name: None            # profiling hook (decode.py sets it)
-        self.fused_attention = False
+        # fused_attention: the location-aware step may run csrc/attention_full.cu; with several heads whether it does is
+        # decided per decode (start(): the kernel's own size query for the beam), and ``fused_step`` records it
+        self.fused_attention = self.fused_step = False
         if fused_attention and self.mode == "loc":
             lay = att.att_layer
             if lay.loc_proj.weight.shape[1] <= 12 and lay.loc_proj.weight.shape[0] % 4 == 0:
                 self.fused_attention = True
-                self._w_conv = lay.loc_conv.weight.detach()[:, 0, :].contiguous()           # [K, 2P+1]
+                w_conv = lay.loc_conv.weight.detach()                                     # [K, H, 2P+1]
+                self._w_conv = w_conv[:, 0, :].contiguous() if self.H == 1 else w_conv.contiguous()
                 self._w_proj = lay.loc_proj.weight.detach().contiguous()
                 self._w_energy = lay.gen_energy.weight.detach().reshape(-1).contiguous()
                 self._b_energy = float(lay.gen_energy.bias.detach().reshape(-1)[0])
@@ -432,15 +436,22 @@ class BatchedStepper:
         u, t, _ = enc.shape
         self.U, self.B, self.T, self.N = u, beam, t, u * beam
         dev = enc.device
-        self.key = torch.tanh(att.proj_k(enc))                                   # [U,T,A]   asr.py:343
-        if self.fused_attention:
-            self.key_t = self.key.transpose(1, 2).contiguous()                   # [U,A,T] channel-major for the fused kernel
-            self.key = None
-        self.value = torch.tanh(att.proj_v(enc)) if att.v_proj else enc          # [U,T,E]
+        if self.H == 1:
+            self.fused_step = self.fused_attention
+            self.key = torch.tanh(att.proj_k(enc))                               # [U,T,A]   asr.py:343
+            if self.fused_attention:
+                self.key_t = self.key.transpose(1, 2).contiguous()               # [U,A,T] channel-major for the fused kernel
+                self.key = None
+            self.value = torch.tanh(att.proj_v(enc)) if att.v_proj else enc      # [U,T,E]
+        else:
+            self._start_heads(enc, beam)
         self.pad = torch.arange(t, device=dev)[None, :] >= enc_len[:, None]      # [U,T]     module.py:1100-1107
         if self.mode == "loc":
             uni = (1.0 / enc_len.to(torch.float32))[:, None].expand(u, t).masked_fill(self.pad, 0.0)   # module.py:1157-1160
-            self.prev_att = uni[:, None, :].expand(u, beam, t).reshape(self.N, t).contiguous()
+            if self.H == 1:
+                self.prev_att = uni[:, None, :].expand(u, beam, t).reshape(self.N, t).contiguous()
+            else:                                                                # [N,H,T]: every head starts uniform
+                self.prev_att = uni[:, None, None, :].expand(u, beam, self.H, t).reshape(self.N, self.H, t).contiguous()
         else:
             self.prev_att = None
         self.dec_fused = isinstance(self.dec, _FusedLstm)
@@ -455,19 +466,34 @@ class BatchedStepper:
             self.lm_state = self.lm_rnn.zeros(self.N, dev) if self.lm_rnn is not None else None
         self._enc_len32 = enc_len.to(torch.int32).contiguous()
 
-    # -- once per decode step ---------------------------------------------------------------
-    def step(self, prev_tok, k=None):
-        """Advance the first ``k`` utterances (all by default).  prev_tok [k*B] long ->
-        (att_logits [k*B,V], lm_logits [k*B,V] | None); the new states are held until
-        :meth:`reorder` commits them in the surviving hypotheses' order."""
-        asr, att = self.asr, self.asr.attention
-        k = self.U if k is None else k
+    def _start_heads(self, enc, beam):
+        """Keys and values of H > 1 heads.  Every head of a hypothesis attends ITS OWN utterance's encoder output: the
+        batch-1 meaning of model.Attention (at batch > 1 its ``value.repeat(num_head, 1, 1)`` would pair heads with other
+        utterances' values, which the per-hypothesis decode never does)."""
+        att, h = self.asr.attention, self.H
+        u, t, _ = enc.shape
+        key = torch.tanh(att.proj_k(enc)).view(u, t, h, -1)                      # [U,T,H,A]  asr.py:343
+        self.fused_step = False
+        if self.fused_attention and enc.is_cuda:
+            from . import ops
+            k_filt, _, width = self._w_conv.shape
+            self.fused_step = ops.attention_loc_heads_supported(beam, h, key.shape[3], k_filt, width)
+        value = torch.tanh(att.proj_v(enc)) if att.v_proj else enc               # [U,T,H*E] or [U,T,E]
+        if self.fused_step:
+            self.key_t, self.key = key.permute(0, 2, 3, 1).contiguous(), None    # [U,H,A,T] channel-major per head
+            self.value = value                                                   # the kernel reads head h's columns in place
+        else:
+            self.key = key.permute(0, 2, 1, 3).contiguous()                      # [U,H,T,A]
+            self.value = value.view(u, t, h, -1).permute(0, 2, 1, 3).contiguous() if att.v_proj else value   # [U,H,T,E]
+
+    def _attend(self, query, k):
+        """The attention step of the first k utterances: query [k*B, H*A] -> (alignments, context [k*B, E])."""
+        att = self.asr.attention
         b, t = self.B, self.T
         n = k * b
-        self._k = k
-        dec_h = self.dec.hidden(n) if self.dec_fused else torch.cat([h[:n] for h in self.dec_state[0]], dim=1)
-        query = torch.tanh(att.proj_q(dec_h))                                              # asr.py:337 / :251-254
-        if self.mode == "loc" and self.fused_attention:
+        if self.H > 1:
+            attn, context = self._attend_heads(query, k)
+        elif self.mode == "loc" and self.fused_attention:
             from . import ops
             # conv + energies + masked softmax + context in one kernel (csrc/attention_full.cu)
             attn, context = ops.attention_loc_full(self.key_t, self.value, query.contiguous(), self.prev_att, self._enc_len32,
@@ -485,6 +511,51 @@ class BatchedStepper:
             score = (energy / self.temperature).masked_fill(self.pad[:k, None, :], -np.inf)
             attn = torch.softmax(score, dim=-1)                                        # [k,B,T]
             context = torch.bmm(attn, self.value[:k]).view(n, -1)                      # module.py:1114
+        return attn, context
+
+    def _attend_heads(self, query, k):
+        """One attention step of H > 1 heads for the first k utterances: (alignments [k*B,H,T], merge_head(context))."""
+        att, h = self.asr.attention, self.H
+        b, t = self.B, self.T
+        n = k * b
+        if self.fused_step:
+            from . import ops
+            # conv over the H alignments + energies + masked softmax + per-head contexts in one kernel (csrc/attention_full.cu)
+            attn, ctx = ops.attention_loc_heads(self.key_t, self.value, query.contiguous(), self.prev_att, self._enc_len32,
+                                                self._w_conv, self._w_proj, self._w_energy, self._b_energy, self.temperature, b,
+                                                att.v_proj, n_run=k)
+        else:
+            q = query.view(k, b, h, -1)
+            if self.mode == "loc":
+                lay = att.att_layer
+                loc = torch.tanh(lay.loc_proj(lay.loc_conv(self.prev_att[:n]).transpose(1, 2))).view(k, b, t, -1)   # shared by the heads
+                # one head at a time: the temporaries stay the size of the single-head step's
+                energy = torch.stack([lay.gen_energy(torch.tanh(self.key[:k, j, None] + q[:, :, j, None, :] + loc)).squeeze(-1)
+                                      for j in range(h)], dim=2)                 # [k,B,H,T]
+            else:
+                energy = torch.matmul(q.transpose(1, 2), self.key[:k].transpose(2, 3)).transpose(1, 2)          # [k,B,H,T]
+            score = (energy / self.temperature).masked_fill(self.pad[:k, None, None, :], -np.inf)
+            attn = torch.softmax(score, dim=-1)                                  # [k,B,H,T]
+            if att.v_proj:
+                ctx = torch.matmul(attn.transpose(1, 2), self.value[:k]).transpose(1, 2)                          # [k,B,H,E]
+            else:
+                ctx = torch.bmm(attn.reshape(k, b * h, t), self.value[:k])       # [k,B*H,E]
+            attn, ctx = attn.reshape(n, h, t), ctx.reshape(n, -1)
+        return attn, F.linear(ctx, att.merge_head.weight, att.merge_head.bias)   # merge_head: [n,H*E] -> [n,E]
+
+    # -- once per decode step ---------------------------------------------------------------
+    def step(self, prev_tok, k=None):
+        """Advance the first ``k`` utterances (all by default).  prev_tok [k*B] long ->
+        (att_logits [k*B,V], lm_logits [k*B,V] | None); the new states are held until
+        :meth:`reorder` commits them in the surviving hypotheses' order."""
+        asr, att = self.asr, self.asr.attention
+        k = self.U if k is None else k
+        b, t = self.B, self.T
+        n = k * b
+        self._k = k
+        dec_h = self.dec.hidden(n) if self.dec_fused else torch.cat([h[:n] for h in self.dec_state[0]], dim=1)
+        query = torch.tanh(att.proj_q(dec_h))                                              # asr.py:337 / :251-254
+        attn, context = self._attend(query, k)
         self.mark("step_attention")
         if self.dec_fused:
             home = self.dec.x0_home(n)                                             # decode.py:114-115
@@ -495,7 +566,7 @@ class BatchedStepper:
             dec_in = torch.cat([asr.pre_embed(prev_tok), context], dim=-1)
             top, self._new_dec = self.dec.step(dec_in, self.dec_state, n)
         att_logits = asr.decoder.char_trans(top)                                   # asr.py:265
-        self._new_att = attn.view(n, t) if self.mode == "loc" else None
+        self._new_att = (attn.view(n, t) if self.H == 1 else attn) if self.mode == "loc" else None
         self.mark("step_speller")
         lm_logits = None
         if self.lm is not None:

@@ -228,6 +228,31 @@ int e2e_attention_loc_full(const float *key_t, const float *value, const float *
                            float b_energy, float temperature, int n_run, int B, int T, int A, int K, int W, int E,
                            int hyps_per_unit, float *attn, float *ctx, void *stream);
 
+/* (f-1, multi-head) The same step for attention.num_head = H heads (model.py Attention / LocationAwareAttention with
+ * num_head > 1, at the batch-1 meaning the per-hypothesis decode gives them), for the first n_run utterances x B beam
+ * slots (hypothesis n = u*B + b):
+ *   feat[n][k][t]  = sum_h sum_j w_conv[k][h][j] * prev_att[n][h][t + j - W/2]     (Conv1d H->K, zero padded, no bias)
+ *   loc[n][t][a]   = tanh(sum_k w_proj[a][k] * feat[n][k][t])                        (shared by all heads)
+ *   attn[n][h][t]  = softmax_t( (b_e + sum_a w_e[a] * tanh(key[u][h][t][a] + query[n][h*A + a] + loc[n][t][a]))
+ *                               / temperature ),  t < enc_len[u];  exactly 0 for t >= enc_len[u]
+ *   ctx[n][h*E+e]  = sum_{t < enc_len[u]} attn[n][h][t] * value_h[u][t][e]
+ *   key_t [U][H][A][T] (tanh(proj_k(enc)) head by head, CHANNEL-major), query [n][H*A] (tanh(proj_q(.)) as is),
+ *   prev_att [n][H][T] (zero beyond enc_len[u]), w_conv [K][H][W], w_proj [A][K], w_energy [A]; attn [n][H][T],
+ *   ctx [n][H*E] (merge_head's input: the caller applies merge_head).
+ *   per_head_values = 0: value [U][T][E], shared by every head (no value projection: each head of a hypothesis attends
+ *   its own utterance's encoder output); 1: value [U][T][H*E] (tanh(proj_v(enc)) as is), value_h = columns h*E..h*E+E-1.
+ *   hyps_per_unit as e2e_attention_loc_full (the result does not depend on it).  H = 1 gives the bits of
+ *   e2e_attention_loc_full.
+ *   Needs 1 <= H <= 4, K <= 12, A % 4 == 0, W odd, B <= 32 and the filters, per-channel constants, one alignment window
+ *   per warp and the queries of at least one group of beam slots within the kernel's shared memory: every such shape is
+ *   accepted by e2e_attention_loc_heads_supported (1 / 0), which callers query before choosing this path; any other
+ *   returns E2E_ERR_UNSUPPORTED before a launch.  Every beam 1..32 with H <= 4 is supported at A = 300, W = 201, K <= 12. */
+int e2e_attention_loc_heads_supported(int B, int H, int A, int K, int W);
+int e2e_attention_loc_heads(const float *key_t, const float *value, const float *query, const float *prev_att,
+                            const int *enc_len, const float *w_conv, const float *w_proj, const float *w_energy,
+                            float b_energy, float temperature, int n_run, int B, int H, int T, int A, int K, int W, int E,
+                            int per_head_values, int hyps_per_unit, float *attn, float *ctx, void *stream);
+
 /* (next, SURVEY §8f row f-2) One-token LSTM step of the batched RNNLM (src/lm.py:27-38: nn.LSTM on a
  * [1,1] token) and speller (src/asr.py:259-266).  The recurrent GEMMs stay library calls on an exact 3-piece
  * bf16 split of the fp32 operands; these two entry points are everything around them.
