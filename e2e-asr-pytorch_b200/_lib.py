@@ -75,12 +75,19 @@ SIGNATURES = {
                                                 c_int, c_float, c_void_p]),
     "e2e_lstm_cell_f16x2": (c_int, [c_void_p, ctypes.c_longlong, c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
                                     c_void_p, c_void_p, c_void_p, ctypes.c_longlong, c_int, c_int, c_float, c_void_p]),
+    "e2e_gru_cell": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                             c_void_p, c_void_p, ctypes.c_longlong, c_int, c_int, c_void_p]),
+    "e2e_gru_cell_f16x2": (c_int, [c_void_p, ctypes.c_longlong, c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                   c_void_p, c_void_p, ctypes.c_longlong, c_int, c_int, c_float, c_void_p]),
     "e2e_conv3x3_unfold_split": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, ctypes.c_longlong, c_int, c_void_p, c_void_p]),
     "e2e_conv_bias_relu_mask": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, ctypes.c_longlong,
                                         ctypes.c_longlong, c_void_p]),
     "e2e_lstm_sequence": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p, c_void_p,
                                   c_int, c_int, c_int, c_int,
                                   c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p]),
+    "e2e_gru_sequence": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p, c_void_p,
+                                 c_int, c_int, c_int, c_int,
+                                 c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "e2e_conv1_direct": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
                                  c_void_p, c_void_p]),
     "e2e_conv_bias_relu_mask_pool": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),

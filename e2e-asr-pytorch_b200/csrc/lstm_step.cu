@@ -8,7 +8,9 @@
 //                            reference's operation order (nn.LSTM cell: src/lm.py:31, src/asr.py:262),
 //                            reading c through the parents' row index, and writing the bf16 split
 //                            of h' into the NEXT layer's A operand
-// Both are pure HBM streams: one pass over their inputs and outputs, 16-byte accesses.
+//   gru_cell_kernel        : the same for an nn.GRU layer (no c state): gates in four blocks [r | z | n_x | n_h]
+//                            (+ bias, + table) -> h' in ATen's GRU cell order, h read through the parents' row index
+// All are pure HBM streams: one pass over their inputs and outputs, 16-byte accesses.
 //
 // Two operand formats (template parameter kPieces):
 //   3 : x == a1 + a2 + a3, bf16 pieces (24 mantissa bits, any magnitude) — six partial GEMM products
@@ -207,6 +209,87 @@ lstm_cell_kernel(const CellParams p)
     }
 }
 
+// GRU step with the gates in four D-wide blocks [r | z | n_x | n_h] (one GEMM chain per layer, like the LSTM: the
+// weight rows of n_x carry only W_in, those of n_h only W_hn, so the two n-gate products stay apart)
+struct GruCellParams {
+    const float *gates; long long gates_pitch; const float *bias; const float *table; const long long *tok;
+    const float *h_prev; const long long *idx; int n, D;
+    float *h_new; unsigned short *a_next; long long a_pitch; int K_next, off_next;
+    float gate_scale, next_scale;        // kPieces == 2: as in CellParams
+};
+
+// ATen's GRU cell order (nn.GRU on the CPU): n = tanh(z_nx + r * z_nh), h' = (h - n) * u + n, every op rounded
+__device__ __forceinline__ float gru_unit(const float (&g)[4], const float (&b)[4], const float *tb, float h)
+{
+    float z[4];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+        z[q] = __fadd_rn(g[q], b[q]);
+        if (tb) z[q] = __fadd_rn(tb[q], z[q]);              // + layer-0 input projection
+    }
+    const float r = sigmoid_f32(z[0]), u = sigmoid_f32(z[1]);
+    const float nn = tanhf(__fadd_rn(z[2], __fmul_rn(r, z[3])));
+    return __fadd_rn(__fmul_rn(__fsub_rn(h, nn), u), nn);
+}
+
+// one thread per (row, kW consecutive hidden units); the sibling of lstm_cell_kernel without the c state
+template <int kW, int kPieces>
+__global__ void __launch_bounds__(256)
+gru_cell_kernel(const GruCellParams p)
+{
+    const int r = blockIdx.y;
+    const float *g = p.gates + (long long)r * p.gates_pitch;
+    const float *tb = p.table ? p.table + p.tok[r] * (long long)(4 * p.D) : nullptr;
+    const long long prow = p.idx ? p.idx[r] : r;
+    const float *hp = p.h_prev + prow * p.D;
+    for (int d = (blockIdx.x * blockDim.x + threadIdx.x) * kW; d < p.D; d += gridDim.x * blockDim.x * kW) {
+        float gv[4][kW], bv[4][kW], tv[4][kW], hv[kW];
+        if (kW == 4) {
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const float4 a = __ldg(reinterpret_cast<const float4 *>(g + q * p.D + d));
+                const float4 b = __ldg(reinterpret_cast<const float4 *>(p.bias + q * p.D + d));
+                gv[q][0] = a.x; gv[q][1] = a.y; gv[q][2] = a.z; gv[q][3] = a.w;
+                bv[q][0] = b.x; bv[q][1] = b.y; bv[q][2] = b.z; bv[q][3] = b.w;
+                if (tb) {
+                    const float4 t = __ldg(reinterpret_cast<const float4 *>(tb + q * p.D + d));
+                    tv[q][0] = t.x; tv[q][1] = t.y; tv[q][2] = t.z; tv[q][3] = t.w;
+                }
+            }
+            const float4 h = __ldg(reinterpret_cast<const float4 *>(hp + d));
+            hv[0] = h.x; hv[1] = h.y; hv[2] = h.z; hv[3] = h.w;
+        } else {
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                gv[q][0] = __ldg(g + q * p.D + d);
+                bv[q][0] = __ldg(p.bias + q * p.D + d);
+                if (tb) tv[q][0] = __ldg(tb + q * p.D + d);
+            }
+            hv[0] = __ldg(hp + d);
+        }
+        float h2[kW];
+#pragma unroll
+        for (int i = 0; i < kW; ++i) {
+            if (kPieces == 2) {
+#pragma unroll
+                for (int q = 0; q < 4; ++q) gv[q][i] = __fmul_rn(gv[q][i], p.gate_scale);
+            }
+            const float gi[4] = {gv[0][i], gv[1][i], gv[2][i], gv[3][i]};
+            const float bi[4] = {bv[0][i], bv[1][i], bv[2][i], bv[3][i]};
+            const float ti[4] = {tb ? tv[0][i] : 0.0f, tb ? tv[1][i] : 0.0f, tb ? tv[2][i] : 0.0f, tb ? tv[3][i] : 0.0f};
+            h2[i] = gru_unit(gi, bi, tb ? ti : nullptr, hv[i]);
+        }
+        float *ho = p.h_new + (long long)r * p.D + d;
+        if (kW == 4) *reinterpret_cast<float4 *>(ho) = make_float4(h2[0], h2[1], h2[2], h2[3]);
+        else ho[0] = h2[0];
+        if (p.a_next) {
+            unsigned short *o = p.a_next + (long long)r * p.a_pitch + p.off_next + d;
+            if constexpr (kW == 4) store_pieces4<kPieces>(h2, p.next_scale, o, p.K_next);
+            else store_pieces1<kPieces>(h2[0], p.next_scale, o, p.K_next);
+        }
+    }
+}
+
 }  // namespace e2e
 
 namespace {
@@ -291,11 +374,12 @@ int split_rows_multi_impl(const char *name, int pieces, float scale, int n_src, 
     return check_launch(name);
 }
 
-int cell_impl(const char *name, int pieces, float gate_scale, float next_scale, const float *gates, long long gates_pitch,
-              const float *bias, const float *table, const long long *tok, const float *c_prev, const long long *row_idx, int n, int D,
+// the LSTM cell (c_new given) or the GRU cell (c_new == nullptr, s_prev = h_prev) over n rows
+int cell_impl(const char *name, bool gru, int pieces, float gate_scale, float next_scale, const float *gates, long long gates_pitch,
+              const float *bias, const float *table, const long long *tok, const float *s_prev, const long long *row_idx, int n, int D,
               float *c_new, float *h_new, void *a_next16, long long a_pitch, int K_next, int off_next, void *stream)
 {
-    if (!gates || !bias || !c_prev || !c_new || !h_new || (table && !tok)) return set_error(E2E_ERR_ARG, "%s: null pointer", name);
+    if (!gates || !bias || !s_prev || (!gru && !c_new) || !h_new || (table && !tok)) return set_error(E2E_ERR_ARG, "%s: null pointer", name);
     if (n <= 0 || D <= 0 || gates_pitch < 4LL * D) return set_error(E2E_ERR_ARG, "%s: bad size", name);
     if (a_next16 && (K_next <= 0 || off_next < 0 || off_next + D > K_next || a_pitch < (long long)pieces * K_next))
         return set_error(E2E_ERR_ARG, "%s: bad next-layer operand geometry", name);
@@ -303,12 +387,12 @@ int cell_impl(const char *name, int pieces, float gate_scale, float next_scale, 
         return set_error(E2E_ERR_ARG, "%s: scales must be powers of two", name);
     CellParams p;
     p.gates = gates; p.gates_pitch = gates_pitch; p.bias = bias; p.table = table; p.tok = tok;
-    p.c_prev = c_prev; p.idx = row_idx; p.D = D; p.a_pitch = a_pitch; p.K_next = K_next; p.off_next = off_next;
+    p.c_prev = s_prev; p.idx = row_idx; p.D = D; p.a_pitch = a_pitch; p.K_next = K_next; p.off_next = off_next;
     p.gate_scale = gate_scale; p.next_scale = next_scale;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const bool vec = (D % 4 == 0) && (gates_pitch % 4 == 0) && !(reinterpret_cast<uintptr_t>(gates) & 15) &&
                      !(reinterpret_cast<uintptr_t>(bias) & 15) && !(reinterpret_cast<uintptr_t>(table) & 15) &&
-                     !(reinterpret_cast<uintptr_t>(c_prev) & 15) && !(reinterpret_cast<uintptr_t>(c_new) & 15) &&
+                     !(reinterpret_cast<uintptr_t>(s_prev) & 15) && !(reinterpret_cast<uintptr_t>(c_new) & 15) &&
                      !(reinterpret_cast<uintptr_t>(h_new) & 15) &&
                      (!a_next16 || ((a_pitch % 4 == 0) && (K_next % 4 == 0) && (off_next % 4 == 0) && !(reinterpret_cast<uintptr_t>(a_next16) & 7)));
     const int per_thread = vec ? 4 : 1;
@@ -320,12 +404,22 @@ int cell_impl(const char *name, int pieces, float gate_scale, float next_scale, 
         p.gates = gates + (long long)r0 * gates_pitch;
         p.tok = tok ? tok + r0 : nullptr;
         p.idx = row_idx ? row_idx + r0 : nullptr;
-        p.c_prev = row_idx ? c_prev : c_prev + (long long)r0 * D;
-        p.c_new = c_new + (long long)r0 * D;
+        p.c_prev = row_idx ? s_prev : s_prev + (long long)r0 * D;
+        p.c_new = gru ? nullptr : c_new + (long long)r0 * D;
         p.h_new = h_new + (long long)r0 * D;
         p.a_next = a_next16 ? static_cast<unsigned short *>(a_next16) + (long long)r0 * a_pitch : nullptr;
         const dim3 grid(bx, rows);
-        if (pieces == 3) {
+        if (gru) {
+            const GruCellParams q{p.gates, p.gates_pitch, p.bias, p.table, p.tok, p.c_prev, p.idx, p.n, p.D,
+                                  p.h_new, p.a_next, p.a_pitch, p.K_next, p.off_next, p.gate_scale, p.next_scale};
+            if (pieces == 3) {
+                if (vec) gru_cell_kernel<4, 3><<<grid, threads, 0, st>>>(q);
+                else gru_cell_kernel<1, 3><<<grid, threads, 0, st>>>(q);
+            } else {
+                if (vec) gru_cell_kernel<4, 2><<<grid, threads, 0, st>>>(q);
+                else gru_cell_kernel<1, 2><<<grid, threads, 0, st>>>(q);
+            }
+        } else if (pieces == 3) {
             if (vec) lstm_cell_kernel<4, 3><<<grid, threads, 0, st>>>(p);
             else lstm_cell_kernel<1, 3><<<grid, threads, 0, st>>>(p);
         } else {
@@ -372,7 +466,7 @@ extern "C" int e2e_lstm_cell(const float *gates, long long gates_pitch, const fl
                              float *c_new, float *h_new, void *a_next_bf16, long long a_pitch, int K_next, int off_next,
                              void *stream)
 {
-    return cell_impl("e2e_lstm_cell", 3, 1.0f, 1.0f, gates, gates_pitch, bias, table, tok, c_prev, row_idx, n, D, c_new, h_new,
+    return cell_impl("e2e_lstm_cell", false, 3, 1.0f, 1.0f, gates, gates_pitch, bias, table, tok, c_prev, row_idx, n, D, c_new, h_new,
                      a_next_bf16, a_pitch, K_next, off_next, stream);
 }
 
@@ -381,6 +475,23 @@ extern "C" int e2e_lstm_cell_f16x2(const float *gates, long long gates_pitch, fl
                                    float *c_new, float *h_new, void *a_next_f16, long long a_pitch, int K_next, int off_next,
                                    float next_scale, void *stream)
 {
-    return cell_impl("e2e_lstm_cell_f16x2", 2, gate_scale, next_scale, gates, gates_pitch, bias, table, tok, c_prev, row_idx, n, D,
+    return cell_impl("e2e_lstm_cell_f16x2", false, 2, gate_scale, next_scale, gates, gates_pitch, bias, table, tok, c_prev, row_idx, n, D,
                      c_new, h_new, a_next_f16, a_pitch, K_next, off_next, stream);
+}
+
+extern "C" int e2e_gru_cell(const float *gates, long long gates_pitch, const float *bias, const float *table, const long long *tok,
+                            const float *h_prev, const long long *row_idx, int n, int D,
+                            float *h_new, void *a_next_bf16, long long a_pitch, int K_next, int off_next, void *stream)
+{
+    return cell_impl("e2e_gru_cell", true, 3, 1.0f, 1.0f, gates, gates_pitch, bias, table, tok, h_prev, row_idx, n, D, nullptr, h_new,
+                     a_next_bf16, a_pitch, K_next, off_next, stream);
+}
+
+extern "C" int e2e_gru_cell_f16x2(const float *gates, long long gates_pitch, float gate_scale, const float *bias, const float *table,
+                                  const long long *tok, const float *h_prev, const long long *row_idx, int n, int D,
+                                  float *h_new, void *a_next_f16, long long a_pitch, int K_next, int off_next, float next_scale,
+                                  void *stream)
+{
+    return cell_impl("e2e_gru_cell_f16x2", true, 2, gate_scale, next_scale, gates, gates_pitch, bias, table, tok, h_prev, row_idx, n, D,
+                     nullptr, h_new, a_next_f16, a_pitch, K_next, off_next, stream);
 }

@@ -284,7 +284,7 @@ class RecurrentLayer(nn.Module):
     # -- packed device path (CUDA only; SURVEY §8f row f-4) ----------------------------------------------
     def packed_supported(self):
         rnn = self.layer
-        return (isinstance(rnn, nn.LSTM) and rnn.num_layers == 1 and self.sample_rate == 1 and not self.layer_norm
+        return (isinstance(rnn, (nn.LSTM, nn.GRU)) and rnn.num_layers == 1 and self.sample_rate == 1 and not self.layer_norm
                 and rnn.hidden_size <= 384)
 
     def _packed_weights(self):
@@ -295,10 +295,20 @@ class RecurrentLayer(nn.Module):
         if key not in cache:
             sfx = ["", "_reverse"] if rnn.bidirectional else [""]
             g = lambda n: getattr(rnn, n).detach().float()
-            w_in = torch.cat([g("weight_ih_l0" + x) for x in sfx], dim=0)                       # [dirs*4H, in]
-            dirs = [((g("bias_ih_l0" + x) + g("bias_hh_l0" + x)).contiguous(),
-                     g("weight_hh_l0" + x).view(4, rnn.hidden_size, rnn.hidden_size).permute(2, 1, 0).contiguous())
-                    for x in sfx]                                                                  # w_t [k][u][gate]
+            h = rnn.hidden_size
+            w_in = torch.cat([g("weight_ih_l0" + x) for x in sfx], dim=0)                       # [dirs*4H (GRU: 3H), in]
+            if isinstance(rnn, nn.LSTM):
+                dirs = [((g("bias_ih_l0" + x) + g("bias_hh_l0" + x)).contiguous(),
+                         g("weight_hh_l0" + x).view(4, h, h).permute(2, 1, 0).contiguous())
+                        for x in sfx]                                                              # w_t [k][u][gate]
+            else:
+                # bias [b_ir+b_hr | b_iz+b_hz | b_in | b_hn]; w_t [k][u][r, z, n, 0] (csrc/lstm_seq.cu, GRU form)
+                dirs = []
+                for x in sfx:
+                    b_ih, b_hh, w_hh = g("bias_ih_l0" + x), g("bias_hh_l0" + x), g("weight_hh_l0" + x).view(3, h, h)
+                    bias = torch.cat([b_ih[:2 * h] + b_hh[:2 * h], b_ih[2 * h:], b_hh[2 * h:]]).contiguous()
+                    w_t = torch.cat([w_hh, w_hh.new_zeros(1, h, h)]).permute(2, 1, 0).contiguous()
+                    dirs.append((bias, w_t))
             pj = (SplitLinear(self.pj.weight.detach().float()), self.pj.bias.detach().float()) if self.proj else None
             cache[key] = (SplitLinear(w_in), dirs, pj)
         return cache[key]
@@ -306,15 +316,17 @@ class RecurrentLayer(nn.Module):
     def forward_packed(self, x, frame_off, lens32, group_first, group_rows):
         """x [F, in]: the valid frames of all utterances back to back (utterance n at rows frame_off[n] ..
         + lens32[n]).  Input projections of both directions are one split-bf16 GEMM over all frames, the
-        recurrence is one persistent kernel launch (csrc/lstm_seq.cu), the projection another GEMM."""
+        recurrence is one persistent kernel launch (csrc/lstm_seq.cu, LSTM or GRU form), the projection another GEMM."""
         from . import ops
         lin_in, dirs, pj = self._packed_weights()
         h = self.layer.hidden_size
-        gates = split_gemm_rows(x.contiguous(), lin_in)                                          # [F, dirs*4H]
+        gru = isinstance(self.layer, nn.GRU)
+        n_gates = 3 if gru else 4
+        gates = split_gemm_rows(x.contiguous(), lin_in)                                          # [F, dirs*n_gates*H]
         out = torch.empty((x.shape[0], h * len(dirs)), dtype=torch.float32, device=x.device)
         fw = (dirs[0][0], dirs[0][1], 0, 0)
-        bw = (dirs[1][0], dirs[1][1], 4 * h, h) if len(dirs) == 2 else None
-        ops.lstm_sequence(gates, out, frame_off, lens32, group_first, group_rows, h, fw, bw)
+        bw = (dirs[1][0], dirs[1][1], n_gates * h, h) if len(dirs) == 2 else None
+        (ops.gru_sequence if gru else ops.lstm_sequence)(gates, out, frame_off, lens32, group_first, group_rows, h, fw, bw)
         if pj is not None:
             out = torch.tanh(split_gemm_rows(out, pj[0]).add_(pj[1]))
         return out

@@ -379,6 +379,37 @@ def lstm_cell(gates, bias, c_prev, row_idx, n, c_new, h_new, table=None, tok=Non
                                             _stream()))
 
 
+def gru_cell(gates, bias, h_prev, row_idx, n, h_new, table=None, tok=None, a_next=None, k_next=0, off_next=0,
+             gate_scale=None, next_scale=None):
+    """Fused GRU cell (see e2e_gru_cell): gates [>=n,4D] fp32 in the blocks [r | z | n_x | n_h] -> h_new [>=n,D] (+ split
+    of h into a_next).  h_prev is read through ``row_idx``.  ``gate_scale`` / ``next_scale`` as in lstm_cell."""
+    _chk(gates, F32, "gates")
+    _chk(bias, F32, "bias")
+    _chk(h_prev, F32, "h_prev")
+    _chk(row_idx, torch.int64, "row_idx", n)
+    _chk(h_new, F32, "h_new")
+    _chk(table, F32, "table")
+    _chk(tok, torch.int64, "tok", n)
+    f16 = gate_scale is not None
+    if a_next is not None and _pieces(a_next, next_scale if f16 else None) != (2 if f16 else 3):
+        raise TypeError("gru_cell: a_next does not match the operand format")
+    d = h_prev.shape[1]
+    if gates.shape[0] < n or gates.shape[1] < 4 * d or h_new.shape[0] < n or bias.numel() < 4 * d:
+        raise ValueError("gru_cell: inconsistent shapes")
+    if h_new.data_ptr() == h_prev.data_ptr():
+        raise ValueError("gru_cell: h_new must not alias h_prev")
+    a_pitch = int(a_next.stride(0)) if a_next is not None else 0
+    if not f16:
+        L.check(L.load().e2e_gru_cell(L.ptr(gates), int(gates.stride(0)), L.ptr(bias), L.ptr(table), L.ptr(tok), L.ptr(h_prev),
+                                     L.ptr(row_idx), int(n), int(d), L.ptr(h_new), L.ptr(a_next),
+                                     a_pitch, int(k_next), int(off_next), _stream()))
+    else:
+        L.check(L.load().e2e_gru_cell_f16x2(L.ptr(gates), int(gates.stride(0)), float(gate_scale), L.ptr(bias), L.ptr(table), L.ptr(tok),
+                                           L.ptr(h_prev), L.ptr(row_idx), int(n), int(d), L.ptr(h_new), L.ptr(a_next),
+                                           a_pitch, int(k_next), int(off_next), float(next_scale if next_scale is not None else 1.0),
+                                           _stream()))
+
+
 def conv3x3_unfold_split(x_nhwc, valid_rows, first_pixel, n_pixels, out, amax=None):
     """Unfold + split of a block of NHWC pixels (see e2e_conv3x3_unfold_split): out bf16 [>=n_pixels, 27*C] (exact 3-piece
     split), or fp16 [>=n_pixels, 18*C] with ``amax`` (int32 [1]: float bits of the input's maximum) for the 2-piece format."""
@@ -431,6 +462,26 @@ def lstm_sequence(gates, out, frame_off, lens, group_first, group_rows, hidden, 
                                       int(lens.numel()), int(hidden), int(group_first.numel()), len(dirs),
                                       L.ptr(fw[0]), L.ptr(fw[1]), int(fw[2]), int(fw[3]),
                                       L.ptr(bw[0]), L.ptr(bw[1]), int(bw[2]), int(bw[3]), _stream()))
+
+
+def gru_sequence(gates, out, frame_off, lens, group_first, group_rows, hidden, fw, bw=None):
+    """Packed (B)GRU recurrence (see e2e_gru_sequence).  gates [F, >=3H*dirs] fp32, out [F, >=H*dirs];
+    fw / bw = (bias [4H] = [b_ir+b_hr | b_iz+b_hz | b_in | b_hn] | None, w_t [H,H,4] (lane 3 zero), gate_off, out_off)."""
+    _chk(gates, F32, "gates")
+    _chk(out, F32, "out")
+    for t, nm in ((frame_off, "frame_off"), (lens, "lens"), (group_first, "group_first"), (group_rows, "group_rows")):
+        _chk(t, I32, nm)
+    dirs = [fw] + ([bw] if bw is not None else [])
+    for b, w, _, _ in dirs:
+        _chk(b, F32, "bias", 4 * hidden)
+        _chk(w, F32, "w_t", 4 * hidden * hidden)
+    if bw is None:
+        bw = (None, None, 0, 0)
+    L.check(L.load().e2e_gru_sequence(L.ptr(gates), int(gates.stride(0)), L.ptr(out), int(out.stride(0)),
+                                     L.ptr(frame_off), L.ptr(lens), L.ptr(group_first), L.ptr(group_rows),
+                                     int(lens.numel()), int(hidden), int(group_first.numel()), len(dirs),
+                                     L.ptr(fw[0]), L.ptr(fw[1]), int(fw[2]), int(fw[3]),
+                                     L.ptr(bw[0]), L.ptr(bw[1]), int(bw[2]), int(bw[3]), _stream()))
 
 
 def conv1_direct(feat, weight, bias, valid_rows, n_freq, amax_out=None):

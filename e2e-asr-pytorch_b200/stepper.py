@@ -32,7 +32,7 @@ PyTorch restatement below runs.  What keeps the step fast without leaving fp32:
   [U*B, T, 300] temporaries and a batched GEMM, and never touches padded frames; multi-head models
   (attention.num_head = H <= 4) run the same kernel's multi-head form followed by merge_head, and fall back to
   a plain PyTorch multi-head step for what that kernel's shape query refuses (and for scaled-dot attention);
-* the LSTM states are never permuted: a step reads them through the parents' row index
+* the LSTM / GRU states are never permuted: a step reads them through the parents' row index
   (``_FusedLstm``), and the encoder runs over packed frames (``model.Encoder.forward_ragged_packed``).
 """
 import numpy as np
@@ -179,18 +179,40 @@ class _Rnn:
         return ([t.index_select(0, idx) for t in h], [t.index_select(0, idx) for t in c] if c is not None else None)
 
 
+def _gru_blocks(w_ih, w_hh, b_ih, b_hh, emb=None):
+    """One nn.GRU layer in the 4-block gate form [r | z | n_x | n_h] of e2e_gru_cell -> (weight, bias, table).
+    Without ``emb``: weight [[W_ir, W_hr], [W_iz, W_hz], [W_in, 0], [0, W_hn]] against [x | h], bias
+    [b_ir+b_hr | b_iz+b_hz | b_in | b_hn], table None.  With the V embeddings ``emb`` of a tabled layer 0: table
+    [E W_ir^T + b_ir | E W_iz^T + b_iz | E W_in^T + b_in | 0] (computed in float64), weight [[W_hr], [W_hz], [0], [W_hn]]
+    against h, bias [b_hr | b_hz | 0 | b_hn].  The zero blocks keep the n-gate products apart (n = tanh(n_x + r * n_h))
+    in one GEMM chain per layer, at the tensor-core cost of an LSTM layer of the same width."""
+    (w_ir, w_iz, w_in), (w_hr, w_hz, w_hn) = w_ih.chunk(3), w_hh.chunk(3)
+    (b_ir, b_iz, b_in), (b_hr, b_hz, b_hn) = b_ih.chunk(3), b_hh.chunk(3)
+    if emb is None:
+        zi, zh = torch.zeros_like(w_in), torch.zeros_like(w_hn)
+        weight = torch.cat([torch.cat([w_ir, w_hr], 1), torch.cat([w_iz, w_hz], 1), torch.cat([w_in, zh], 1), torch.cat([zi, w_hn], 1)])
+        return weight, torch.cat([b_ir + b_hr, b_iz + b_hz, b_in, b_hn]), None
+    proj = emb.double() @ w_ih.double().t() + b_ih.double()                               # [V, 3D]
+    table = torch.cat([proj, proj.new_zeros(proj.shape[0], w_hh.shape[1])], 1).to(w_ih.dtype)
+    return torch.cat([w_hr, w_hz, torch.zeros_like(w_hn), w_hn]), torch.cat([b_hr, b_hz, torch.zeros_like(b_hn), b_hn]), table
+
+
 class _FusedLstm:
-    """n-layer LSTM advanced one token at a time for a batch of rows, entirely on the device path
+    """n-layer LSTM or GRU advanced one token at a time for a batch of rows, entirely on the device path
     (SURVEY §8f row f-2): per layer one hand-written split kernel, the three split GEMMs (library,
     tensor cores, fp32 accumulation) and one hand-written cell kernel (csrc/lstm_step.cu).  States
     are never permuted: a step reads the previous states through the parents' row index ``idx``
-    and writes the new ones to the other half of a ping-pong buffer.
+    and writes the new ones to the other half of a ping-pong buffer.  A GRU layer uses the same
+    [n, 4D] accumulator through the 4-block gate form of ``_gru_blocks`` and has no c state.
 
     ``split`` selects the GEMM operand format: "bf16x3" (exact 3-piece bf16 split, six partial products, any operand
     range) or "fp16x2" (2-piece fp16 split, three partial products; needs a tabled layer 0 so that every GEMM input
     is a hidden state, |h| <= 1 — the RNNLM, src/lm.py:27-38)."""
 
     def __init__(self, rnn, first_input_table=None, split="bf16x3"):
+        if not isinstance(rnn, (torch.nn.LSTM, torch.nn.GRU)):
+            raise NotImplementedError("only LSTM / GRU recurrent layers are supported")
+        self.gru = isinstance(rnn, torch.nn.GRU)
         if split not in ("bf16x3", "fp16x2"):
             raise ValueError("unknown split format " + str(split))
         if split == "fp16x2" and first_input_table is None:
@@ -202,7 +224,15 @@ class _FusedLstm:
         for l in range(self.layers):
             w_ih, w_hh, b_ih, b_hh = (getattr(rnn, "{}_l{}".format(k, l)).detach().float()
                                       for k in ("weight_ih", "weight_hh", "bias_ih", "bias_hh"))
-            if l == 0 and first_input_table is not None:
+            tabled = l == 0 and first_input_table is not None
+            if self.gru:
+                weight, bias, table = _gru_blocks(w_ih, w_hh, b_ih, b_hh, first_input_table if tabled else None)
+                if tabled:
+                    self.table0 = table.contiguous()
+                self.lin.append(make_lin(weight))
+                self.bias.append(bias.contiguous())
+                self.k_in.append(0 if tabled else w_ih.shape[1])
+            elif tabled:
                 # layer 0 sees one of V embeddings: its input projection is a [V, 4D] table
                 self.table0 = (first_input_table.double() @ w_ih.double().t() + b_ih.double()).float().contiguous()
                 self.lin.append(make_lin(w_hh))
@@ -228,14 +258,15 @@ class _FusedLstm:
             # same buffers as the last decode (and the graphs captured over them): only the initial states are reset
             for l in range(self.layers):
                 self.h[0][l][:n].zero_()
-                self.c[0][l][:n].zero_()
+                if self.c is not None:
+                    self.c[0][l][:n].zero_()
             self.idx = self.idx_buf[:n]
             self.idx_buf.copy_(self._arange)
             self.cur = 0
             return
         self.cap, self.device, self.graphs = n, device, {}
         self.h = [[torch.zeros(n, d, device=device) for _ in range(self.layers)] for _ in range(2)]
-        self.c = [[torch.zeros(n, d, device=device) for _ in range(self.layers)] for _ in range(2)]
+        self.c = None if self.gru else [[torch.zeros(n, d, device=device) for _ in range(self.layers)] for _ in range(2)]
         pieces, a_dtype = (2, torch.float16) if self.f16 else (3, torch.bfloat16)
         self.a = [torch.empty(n, pieces * (self.k_in[l] + d), dtype=a_dtype, device=device) for l in range(self.layers)]
         self.gates = torch.empty(n, 4 * d, device=device)          # GEMM accumulator, reused by every layer
@@ -324,10 +355,13 @@ class _FusedLstm:
                 torch.addmm(y, a[:, :2 * k], lin.b1, out_dtype=torch.float32, out=y)
             torch.addmm(y, a[:, :k], lin.b0, out_dtype=torch.float32, out=y)
             nxt = l + 1 < self.layers
-            ops.lstm_cell(y, self.bias[l], self.c[cur][l], idx, n, self.c[new][l], self.h[new][l],
-                          table=self.table0 if l == 0 else None, tok=tok if (l == 0 and self.table0 is not None) else None,
-                          a_next=self.a[l + 1] if nxt else None, k_next=(self.k_in[l + 1] + d) if nxt else 0, off_next=0,
-                          gate_scale=lin.out_scale if self.f16 else None, next_scale=self.scale)
+            tail = dict(table=self.table0 if l == 0 else None, tok=tok if (l == 0 and self.table0 is not None) else None,
+                        a_next=self.a[l + 1] if nxt else None, k_next=(self.k_in[l + 1] + d) if nxt else 0, off_next=0,
+                        gate_scale=lin.out_scale if self.f16 else None, next_scale=self.scale)
+            if self.gru:
+                ops.gru_cell(y, self.bias[l], self.h[cur][l], idx, n, self.h[new][l], **tail)
+            else:
+                ops.lstm_cell(y, self.bias[l], self.c[cur][l], idx, n, self.c[new][l], self.h[new][l], **tail)
         self.cur = new
         return self.h[new][self.layers - 1][:n]
 
@@ -347,11 +381,11 @@ class BatchedStepper:
         self.vgg_split = vgg_split               # their operand format
         self.mode, self.temperature = att.mode, att.att_layer.temperature
         self.H = att.num_head
-        # fused device LSTM steps (csrc/lstm_step.cu) whenever the weights live on a GPU; the plain
-        # PyTorch cells otherwise (CPU tests of the host logic, GRU models)
+        # fused device LSTM / GRU steps (csrc/lstm_step.cu) whenever the weights live on a GPU; the plain
+        # PyTorch cells otherwise (CPU tests of the host logic, split_gemm = False)
         def make(rnn, table=None, split="bf16x3"):
             on_gpu = next(rnn.parameters()).is_cuda
-            if split_gemm and on_gpu and isinstance(rnn, torch.nn.LSTM):
+            if split_gemm and on_gpu and isinstance(rnn, (torch.nn.LSTM, torch.nn.GRU)):
                 return _FusedLstm(rnn, table, split)
             return _Rnn(rnn, split_gemm, table)
         self.dec = make(asr.decoder.layers)                  # speller inputs (embedding, context) have no fixed range: bf16x3

@@ -302,6 +302,22 @@ int e2e_lstm_cell_f16x2(const float *gates, long long gates_pitch, float gate_sc
                         float *c_new, float *h_new, void *a_next_f16, long long a_pitch, int K_next, int off_next,
                         float next_scale, void *stream);
 
+/* One-token GRU step (nn.GRU; src/lm.py:5-38 and src/asr.py:183-270 with module: GRU), the sibling of e2e_lstm_cell.
+ * The caller's GEMM produces four D-wide gate blocks [r | z | n_x | n_h] per row: for a layer with input x the weight is
+ * [[W_ir, W_hr], [W_iz, W_hz], [W_in, 0], [0, W_hn]] against A = [x | h] and bias = [b_ir+b_hr | b_iz+b_hz | b_in | b_hn];
+ * for a tabled layer 0 the table row is [E W_ir^T + b_ir | E W_iz^T + b_iz | E W_in^T + b_in | 0], the weight
+ * [[W_hr], [W_hz], [0], [W_hn]] and bias = [b_hr | b_hz | 0 | b_hn].  With z_q = gates[r][q] + bias_q (+ table[tok[r]][q]):
+ *   r = sigmoid(z_r);  u = sigmoid(z_z);  n = tanh(z_nx + r * z_nh);  h'[r] = (h_prev[row(r)] - n) * u + n
+ *   (fp32, every product and sum rounded separately, ATen's CPU GRU cell order), and, if a_next is given, the split of
+ *   h'[r] into the next layer's A operand exactly as e2e_lstm_cell writes it.  h_prev [*][D]; h_new [n][D] (not h_prev).
+ * e2e_gru_cell_f16x2 takes gate_scale / next_scale as e2e_lstm_cell_f16x2 does (|h| < 1 holds for a GRU state too). */
+int e2e_gru_cell(const float *gates, long long gates_pitch, const float *bias, const float *table, const long long *tok,
+                 const float *h_prev, const long long *row_idx, int n, int D,
+                 float *h_new, void *a_next_bf16, long long a_pitch, int K_next, int off_next, void *stream);
+int e2e_gru_cell_f16x2(const float *gates, long long gates_pitch, float gate_scale, const float *bias, const float *table,
+                       const long long *tok, const float *h_prev, const long long *row_idx, int n, int D,
+                       float *h_new, void *a_next_f16, long long a_pitch, int K_next, int off_next, float next_scale, void *stream);
+
 /* (next, SURVEY §8f row f-4) 3x3 "same" convolutions of the VGG front end (src/module.py:672-686) as
  * fp32-accurate tensor-core GEMMs: unfold a block of NHWC pixels into the GEMM's A operand as the exact
  * 3-piece bf16 split [a1 | a2 | a3] of every fp32 value,
@@ -332,6 +348,19 @@ int e2e_lstm_sequence(const float *gates, long long gates_pitch, float *out, lon
                       const float *bias_fw, const float *w_t_fw, int gate_off_fw, int out_off_fw,
                       const float *bias_bw, const float *w_t_bw, int gate_off_bw, int out_off_bw,
                       void *stream);
+
+/* e2e_lstm_sequence for an nn.GRU layer (RNNLayer with module: GRU), same packing, grouping and limits:
+ *   z_{r,z,nx} = gates[frame_off[n] + t][gate_off_d : gate_off_d + 3H] + bias_d[0 : 3H]             (gate order r,z,n)
+ *   z_nh = bias_d[3H : 4H] + W_hn h_prev;  r = sigmoid(z_r + W_hr h_prev);  u = sigmoid(z_z + W_hz h_prev)
+ *   n = tanh(z_nx + r * z_nh);  h = (h_prev - n) * u + n;  out[frame_off[n] + t][out_off_d : +H] = h
+ *   bias_d [4H] = [b_ir + b_hr | b_iz + b_hz | b_in | b_hn] (the 3H input-side bias followed by b_hn; or NULL);
+ *   w_t_d [H][H][4] with w_t[k][u][g] = W_hh[g*H + u][k] for g < 3 and w_t[k][u][3] = 0;  gates_pitch >= 3H. */
+int e2e_gru_sequence(const float *gates, long long gates_pitch, float *out, long long out_pitch,
+                     const int *frame_off, const int *lens, const int *group_first, const int *group_rows,
+                     int N, int H, int n_groups, int n_dirs,
+                     const float *bias_fw, const float *w_t_fw, int gate_off_fw, int out_off_fw,
+                     const float *bias_bw, const float *w_t_bw, int gate_off_bw, int out_off_bw,
+                     void *stream);
 
 /* First VGG layer (Conv2d Cin->Cout 3x3 "same" + bias + ReLU, src/module.py:672-674) straight from the feature
  * frames: feat [N][L][Cin*F] (a frame is Cin blocks of F bins, src/module.py:688-690; row pitch of an utterance
