@@ -82,6 +82,8 @@ SIGNATURES = {
     "e2e_conv3x3_unfold_split": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, ctypes.c_longlong, c_int, c_void_p, c_void_p]),
     "e2e_conv_bias_relu_mask": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, ctypes.c_longlong,
                                         ctypes.c_longlong, c_void_p]),
+    "e2e_conv3x3_igemm_supported": (c_int, [c_int, c_int]),
+    "e2e_conv3x3_igemm": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "e2e_lstm_sequence": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p, c_void_p,
                                   c_int, c_int, c_int, c_int,
                                   c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p]),

@@ -328,7 +328,7 @@ typedef void (*PrefixKernel)(PrefixParams, CUtensorMap);
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
                                   const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn tensor_map_encoder()
+EncodeTiledFn tensor_map_encoder()   // also used by conv_igemm.cu
 {
     static EncodeTiledFn fn = nullptr;
     static bool tried = false;

@@ -139,6 +139,9 @@ class BeamDecoder(nn.Module):
         # the same choice for the VGG convolutions (their activations have no fixed range: the scale is chosen on
         # the device from the running maximum of every layer's input, csrc/conv_split.cu)
         self.vgg_split = os.environ.get("E2E_VGG_SPLIT", "bf16x3")
+        # bf16x3 VGG convolutions: "igemm" runs the 128-channel layer as one tcgen05 implicit GEMM (csrc/conv_igemm.cu),
+        # "unfold" every layer as unfold + three library GEMMs + epilogue kernel (model.VGGFrontEnd.conv_path); same bits
+        self.vgg_conv = "igemm"
         self.fused_attention = True     # hand-written location-aware attention kernel (csrc/attention_full.cu)
         # replay the LSTM stacks of a decode step from CUDA graphs when few utterances are live (stepper._FusedLstm): the tail of a
         # decode is bound by the host's launch rate
@@ -302,11 +305,11 @@ class BeamDecoder(nn.Module):
 
         with _Fp32Math():
             mark("start", True)
-            knobs = (self.split_gemm, self.fused_attention, self.lm_split, self.vgg_split, self.step_graphs)
+            knobs = (self.split_gemm, self.fused_attention, self.lm_split, self.vgg_split, self.step_graphs, self.vgg_conv)
             if self._stepper is None or self._stepper[0] != dev or self._stepper[1] != knobs:
                 self._stepper = (dev, knobs, BatchedStepper(self.asr, self.lm if self.apply_lm else None,
                                                             self.split_gemm, self.fused_attention, self.lm_split, self.vgg_split,
-                                                            self.step_graphs))
+                                                            self.step_graphs, self.vgg_conv))
             stepper = self._stepper[2]
             stepper.mark = mark
             enc, enc_len = stepper.encode(audio_feature, feature_len.to(dev))

@@ -139,6 +139,12 @@ class VGGFrontEnd(nn.Module):
     A_BYTES = 3 << 30      # budget of the unfolded bf16 operand per GEMM block
 
     conv_split_format = "bf16x3"     # "fp16x2": 2-piece fp16 operands, scale per layer input chosen on the device (csrc/conv_split.cu)
+    # bf16x3 layers: "igemm" runs the layers with at most IGEMM_MAX_COUT output channels as one tcgen05 implicit split GEMM
+    # with the epilogue fused (csrc/conv_igemm.cu, bit-equal to the unfold path); "unfold": every layer as unfold+split ->
+    # three library GEMMs -> epilogue kernel.  The 256-channel layers stay on the library either way: at N = 256 its GEMMs
+    # run the split products at 1.1-1.2 PFLOP/s, the implicit GEMM at 0.6 (at N = 128 the library reaches 0.65), DESIGN §4.
+    conv_path = "igemm"
+    IGEMM_MAX_COUT = 128
 
     def _split_weights(self, conv):
         """[9*Cin, Cout] GEMM weights of a 3x3 convolution as the operand stacks of stepper.SplitLinear /
@@ -151,6 +157,15 @@ class VGGFrontEnd(nn.Module):
             cache[key] = SplitLinearF16(w2d, act_scale=1.0) if self.conv_split_format == "fp16x2" else SplitLinear(w2d)
         return cache[key]
 
+    def _igemm_weights(self, conv):
+        """[3, Cout, 9*Cin] bf16: the pieces w1, w2, w3 of _split_weights' SplitLinear, K-major, for e2e_conv3x3_igemm."""
+        cache = self.__dict__.setdefault("_split_cache", {})
+        key = (id(conv), conv.weight.device, "igemm")
+        if key not in cache:
+            lin, k = self._split_weights(conv), 9 * conv.in_channels
+            cache[key] = torch.stack([lin.b0.t(), lin.b1[:k].t(), lin.b2[:k].t()]).contiguous()
+        return cache[key]
+
     def _conv_split(self, x, valid, conv, pool=False, amax_in=None, amax_out=None):
         """x [N,H,W,C] fp32 NHWC, valid [N] int32 -> relu(conv(x) + b) [N,H,W,Cout] NHWC, rows >= valid zeroed;
         with ``pool`` the 2x2 ceil-mode max pooling that follows is fused into the epilogue kernel.
@@ -158,6 +173,10 @@ class VGGFrontEnd(nn.Module):
         operand comes from amax_in, the maximum of its output goes to amax_out."""
         from . import ops
         n, h, w, c = x.shape
+        bias = conv.bias.detach().float().contiguous()
+        if (amax_in is None and self.conv_path == "igemm" and conv.out_channels <= self.IGEMM_MAX_COUT
+                and ops.conv3x3_igemm_supported(c, conv.out_channels)):
+            return ops.conv3x3_igemm(x, valid, self._igemm_weights(conv), bias, "pool" if pool else "relu")
         k = 9 * c
         lin = self._split_weights(conv)
         total = n * h * w
@@ -177,7 +196,6 @@ class VGGFrontEnd(nn.Module):
                 torch.addmm(ym, am[:, :2 * k], lin.b1, out_dtype=torch.float32, out=ym)    # + a1w2 + a2w1
             torch.addmm(ym, am[:, :k], lin.b0, out_dtype=torch.float32, out=ym)            # + a1w1
         y = y.view(n, h, w, conv.out_channels)
-        bias = conv.bias.detach().float().contiguous()
         scale_args = (amax_in, lin.out_scale, amax_out) if f16 else ()
         if pool:
             return ops.conv_bias_relu_mask_pool(y, bias, valid, *scale_args)

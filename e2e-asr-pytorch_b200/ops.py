@@ -427,6 +427,42 @@ def conv3x3_unfold_split(x_nhwc, valid_rows, first_pixel, n_pixels, out, amax=No
                                                        L.ptr(amax), L.ptr(out), _stream()))
 
 
+def conv3x3_igemm_supported(c_in, c_out):
+    """Whether e2e_conv3x3_igemm takes this layer shape."""
+    return bool(L.load().e2e_conv3x3_igemm_supported(int(c_in), int(c_out)))
+
+
+IGEMM_EPILOGUE = {"raw": 0, "relu": 1, "pool": 2}
+
+
+def conv3x3_igemm(x_nhwc, valid_rows, w_split, bias, epilogue="relu"):
+    """3x3 "same" convolution as one tcgen05 implicit split GEMM (see e2e_conv3x3_igemm): x [N,H,W,C] fp32 NHWC,
+    w_split bf16 [3, Cout, 9C] (the pieces of weight.permute(0,2,3,1).reshape(Cout, 9C)).  ``epilogue``: "raw" -> the
+    GEMM result [N*H*W, Cout]; "relu" -> relu(y + bias) masked to rows h < valid_rows[n], [N,H,W,Cout]; "pool" -> its
+    2x2 ceil-mode max pool [N,ceil(H/2),ceil(W/2),Cout]."""
+    _chk(x_nhwc, F32, "x_nhwc")
+    _chk(valid_rows, I32, "valid_rows", x_nhwc.shape[0])
+    _chk(w_split, torch.bfloat16, "w_split")
+    n, h, w, c = x_nhwc.shape
+    if w_split.dim() != 3 or w_split.shape[0] != 3 or w_split.shape[2] != 9 * c:
+        raise ValueError("w_split must be [3, Cout, 9*%d], got %s" % (c, tuple(w_split.shape)))
+    cout = w_split.shape[1]
+    if epilogue not in IGEMM_EPILOGUE:
+        raise ValueError("unknown epilogue " + str(epilogue))
+    if epilogue != "raw":
+        _chk(bias, F32, "bias", cout)
+    if epilogue == "raw":
+        out = torch.empty((n * h * w, cout), dtype=F32, device=x_nhwc.device)
+    elif epilogue == "relu":
+        out = torch.empty((n, h, w, cout), dtype=F32, device=x_nhwc.device)
+    else:
+        out = torch.empty((n, (h + 1) // 2, (w + 1) // 2, cout), dtype=F32, device=x_nhwc.device)
+    L.check(L.load().e2e_conv3x3_igemm(L.ptr(x_nhwc), L.ptr(valid_rows), n, h, w, c, L.ptr(w_split),
+                                      L.ptr(bias) if epilogue != "raw" else None, int(cout), IGEMM_EPILOGUE[epilogue],
+                                      L.ptr(out), _stream()))
+    return out
+
+
 def conv_bias_relu_mask(y_nhwc, bias, valid_rows, amax_in=None, inv_w_scale=None, amax_out=None):
     """In place: y = relu(y + bias) on rows h < valid_rows[n], 0 elsewhere; y [N,H,W,C] NHWC.  With ``amax_in`` (the scale
     word of the layer's INPUT) y is an fp16x2 GEMM result: it is first multiplied by inv_w_scale / act_scale(amax_in);

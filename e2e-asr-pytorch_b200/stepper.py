@@ -370,7 +370,8 @@ class _FusedLstm:
 
 
 class BatchedStepper:
-    def __init__(self, asr, lm=None, split_gemm=False, fused_attention=False, lm_split="bf16x3", vgg_split="bf16x3", step_graphs=False):
+    def __init__(self, asr, lm=None, split_gemm=False, fused_attention=False, lm_split="bf16x3", vgg_split="bf16x3", step_graphs=False,
+                 vgg_conv="igemm"):
         att = asr.attention
         if att.mode not in ("loc", "dot"):
             raise NotImplementedError("attention mode " + str(att.mode))
@@ -379,6 +380,9 @@ class BatchedStepper:
         if vgg_split not in ("bf16x3", "fp16x2"):
             raise ValueError("unknown split format " + str(vgg_split))
         self.vgg_split = vgg_split               # their operand format
+        if vgg_conv not in ("igemm", "unfold"):
+            raise ValueError("unknown VGG convolution path " + str(vgg_conv))
+        self.vgg_conv = vgg_conv                 # and kernel path (model.VGGFrontEnd.conv_path)
         self.mode, self.temperature = att.mode, att.att_layer.temperature
         self.H = att.num_head
         # fused device LSTM / GRU steps (csrc/lstm_step.cu) whenever the weights live on a GPU; the plain
@@ -417,6 +421,7 @@ class BatchedStepper:
         for layer in getattr(enc_mod, "layers", []):
             if hasattr(layer, "conv_split_format"):
                 layer.conv_split_format = self.vgg_split
+                layer.conv_path = self.vgg_conv
         packed = (n_utts > 1 and self.split_conv and feats.is_cuda and hasattr(enc_mod, "forward_ragged_packed")
                   and enc_mod.packed_supported())
         ready = getattr(enc_mod, "chunk_ready", None)

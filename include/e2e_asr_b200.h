@@ -333,6 +333,19 @@ int e2e_conv3x3_unfold_split(const float *in_nhwc, const int *valid_rows, int N,
 int e2e_conv_bias_relu_mask(float *y_nhwc, const float *bias, const int *valid_rows, int N, int H, int W, int C,
                             long long first_pixel, long long n_pixels, void *stream);
 
+/* The same convolution as ONE implicit split GEMM on the tcgen05 tensor cores (csrc/conv_igemm.cu, built into
+ * libe2e_asr_b200_tc.so, which this library links against and loads from its own directory): the A operand is
+ * split from the NHWC input on the way into shared memory (no unfolded operand), the six partial products run into
+ * three fp32 accumulators in the K order of the library GEMMs, and the epilogue of the unfold path is fused, so the
+ * result equals unfold + mm/addmm/addmm + e2e_conv_bias_relu_mask(_pool) bit for bit.
+ *   w_split_bf16 [3][Cout][9C] = the bf16 pieces w1, w2, w3 of Wmat^T (stepper.SplitLinear's split), 16-byte aligned;
+ *   epilogue 0: out [N*H*W][Cout] = the raw GEMM result y;  1: out [N][H][W][Cout] = relu(y + bias), 0 on rows
+ *   h >= valid_rows[n];  2: out [N][ceil(H/2)][ceil(W/2)][Cout] = the 2x2 ceil-mode max pool of that.
+ * Shapes outside e2e_conv3x3_igemm_supported (C and Cout in {128, 256}) return E2E_ERR_UNSUPPORTED before a launch. */
+int e2e_conv3x3_igemm_supported(int C, int Cout);
+int e2e_conv3x3_igemm(const float *in_nhwc, const int *valid_rows, int N, int H, int W, int C,
+                      const void *w_split_bf16, const float *bias, int Cout, int epilogue, float *out, void *stream);
+
 /* (next, SURVEY §8f row f-4) Whole-sequence LSTM recurrence of an encoder layer (RNNLayer, src/module.py:1003-1081:
  * nn.LSTM, optionally bidirectional) over PACKED utterances, one persistent launch per layer:
  *   for every utterance n, direction d and its frames t in walking order (d = 0: 0..len-1, d = 1: len-1..0)
