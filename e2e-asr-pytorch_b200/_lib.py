@@ -90,6 +90,8 @@ SIGNATURES = {
     "e2e_gru_sequence": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p, c_void_p,
                                  c_int, c_int, c_int, c_int,
                                  c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p]),
+    "e2e_packed_subsample_ln": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p,
+                                        c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_void_p]),
     "e2e_conv1_direct": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
                                  c_void_p, c_void_p]),
     "e2e_conv_bias_relu_mask_pool": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),

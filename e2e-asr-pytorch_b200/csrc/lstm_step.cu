@@ -310,7 +310,7 @@ int split_rows_impl(const char *name, int pieces, float scale, const float *src,
     if (n <= 0 || w <= 0 || K <= 0 || off < 0 || off + w > K || dst_pitch < (long long)pieces * K || src_pitch < w)
         return set_error(E2E_ERR_ARG, "%s: bad size", name);
     if (pieces == 2 && !valid_scale(scale)) return set_error(E2E_ERR_ARG, "%s: scale must be a power of two", name);
-    if (n > 65535 * 16) return set_error(E2E_ERR_UNSUPPORTED, "%s: too many rows", name);
+    if (n > 65535 * 16) return set_error(E2E_ERR_UNSUPPORTED, "%s: too many rows", name);   // model.SPLIT_MAX_ROWS
     const bool vec = (w % 4 == 0) && (src_pitch % 4 == 0) && (dst_pitch % 4 == 0) && (K % 4 == 0) && (off % 4 == 0) &&
                      !(reinterpret_cast<uintptr_t>(src) & 15) && !(reinterpret_cast<uintptr_t>(dst16) & 7);
     const int per_thread = vec ? 4 : 1;

@@ -59,16 +59,22 @@ def reference_init_(module):
             raise NotImplementedError
 
 
+# rows one e2e_lstm_split_rows launch takes: must equal the limit split_rows_impl checks (csrc/lstm_step.cu, its grid
+# limit); tests/test_encoder_subsample_host.py holds the two together
+SPLIT_MAX_ROWS = 65535 * 16
+
+
 def split_gemm_rows(x, lin, a_bytes=3 << 30):
     """y = x @ W^T (no bias) as fp32-accurate bf16 tensor-core GEMMs: x [F, K] fp32 (contiguous, CUDA),
     ``lin`` a stepper.SplitLinear holding the weight's three operand stacks.  The exact 3-piece split of a
     block of rows is written by one hand-written kernel (csrc/lstm_step.cu), the three GEMMs accumulate in
-    place; row blocks bound the size of the bf16 operand."""
+    place; row blocks bound the size of the bf16 operand and the split kernel's row count (narrow inputs such
+    as 160 feature bins without a front end reach the latter first)."""
     from . import ops
     f, k = x.shape
     m_out = lin.b0.shape[1]
     y = torch.empty((f, m_out), dtype=torch.float32, device=x.device)
-    blk = max(1, min(f, a_bytes // (3 * k * 2)))
+    blk = max(1, min(f, a_bytes // (3 * k * 2), SPLIT_MAX_ROWS))
     a = torch.empty((blk, 3 * k), dtype=torch.bfloat16, device=x.device)
     for r0 in range(0, f, blk):
         m = min(blk, f - r0)
@@ -302,8 +308,7 @@ class RecurrentLayer(nn.Module):
     # -- packed device path (CUDA only; SURVEY §8f row f-4) ----------------------------------------------
     def packed_supported(self):
         rnn = self.layer
-        return (isinstance(rnn, (nn.LSTM, nn.GRU)) and rnn.num_layers == 1 and self.sample_rate == 1 and not self.layer_norm
-                and rnn.hidden_size <= 384)
+        return isinstance(rnn, (nn.LSTM, nn.GRU)) and rnn.num_layers == 1 and rnn.hidden_size <= 384
 
     def _packed_weights(self):
         from .stepper import SplitLinear
@@ -331,10 +336,12 @@ class RecurrentLayer(nn.Module):
             cache[key] = (SplitLinear(w_in), dirs, pj)
         return cache[key]
 
-    def forward_packed(self, x, frame_off, lens32, group_first, group_rows):
+    def forward_packed(self, x, frame_off, lens32, group_first, group_rows, out_lens=None):
         """x [F, in]: the valid frames of all utterances back to back (utterance n at rows frame_off[n] ..
         + lens32[n]).  Input projections of both directions are one split-bf16 GEMM over all frames, the
-        recurrence is one persistent kernel launch (csrc/lstm_seq.cu, LSTM or GRU form), the projection another GEMM."""
+        recurrence is one persistent kernel launch (csrc/lstm_seq.cu, LSTM or GRU form), LayerNorm and sub-sampling
+        one gather kernel (csrc/encoder_post.cu), the projection another GEMM.  A sub-sampling layer needs
+        ``out_lens``: the host frame counts P' of its output (subsample_lengths); its output is packed back to back."""
         from . import ops
         lin_in, dirs, pj = self._packed_weights()
         h = self.layer.hidden_size
@@ -345,9 +352,54 @@ class RecurrentLayer(nn.Module):
         fw = (dirs[0][0], dirs[0][1], 0, 0)
         bw = (dirs[1][0], dirs[1][1], n_gates * h, h) if len(dirs) == 2 else None
         (ops.gru_sequence if gru else ops.lstm_sequence)(gates, out, frame_off, lens32, group_first, group_rows, h, fw, bw)
+        if self.layer_norm or self.sample_rate > 1:
+            out = self._packed_post(out, frame_off, lens32, out_lens)
         if pj is not None:
             out = torch.tanh(split_gemm_rows(out, pj[0]).add_(pj[1]))
         return out
+
+    def _packed_post(self, out, frame_off, lens32, out_lens):
+        """_post's LayerNorm and sub-sampling (dropout is the identity in eval) on packed frames."""
+        from . import ops
+        r = self.sample_rate
+        if r == 1:
+            out_off, out_len, n_out = frame_off, lens32, out.shape[0]
+        else:
+            if out_lens is None:
+                raise ValueError("forward_packed: a sub-sampling layer needs out_lens, the frame counts of its output")
+            out_off, out_len = packed_offsets(out_lens, out.device)
+            n_out = int(out_lens.sum())
+        ln = self.ln if self.layer_norm else None
+        f32 = lambda t: None if t is None else t.detach().float().contiguous()
+        return ops.packed_subsample_ln(out, frame_off, out_off, out_len, n_out, stride=r,
+                                       g=r if self.sample_style == "concat" else 1, weight=f32(ln.weight) if ln else None,
+                                       bias=f32(ln.bias) if ln else None, eps=ln.eps if ln else 1e-5)
+
+
+def subsample_lengths(p, x, sample_rate, sample_style):
+    """Frame counts after a recurrent layer's sub-sampling, as a batch-1 call of RecurrentLayer produces them: p (P) the
+    frames that physically exist and that the next layer's recurrence walks, x (X) the reported x_len; 1-D integer
+    tensors, one entry per utterance.  'drop' keeps frames 0, r, 2r, .. of the P: ceil(P / r); 'concat' makes rows of
+    r consecutive frames and crops the P % r left over: P // r.  X becomes X // r either way, so a 'drop' layer that
+    meets an odd P leaves P' > X'.  Raises ValueError for an utterance left without frames (the reference cannot encode
+    it either)."""
+    p, x = torch.as_tensor(p).reshape(-1), torch.as_tensor(x).reshape(-1)
+    if sample_rate == 1:
+        return p, x
+    r = int(sample_rate)
+    p2 = (p + r - 1) // r if sample_style == "drop" else p // r
+    empty = (p2 < 1).nonzero().reshape(-1)
+    if len(empty):
+        i = int(empty[0])
+        raise ValueError("utterance %d: its %d encoder frames leave none after '%s' sub-sampling by %d" % (i, int(p[i]), sample_style, r))
+    return p2, x // r
+
+
+def packed_offsets(lens_host, device):
+    """(frame_off, lens) int32 device tensors of utterances of lens_host frames packed back to back."""
+    t = torch.as_tensor(lens_host).long().reshape(-1)
+    off = torch.cumsum(t, 0) - t
+    return off.to(torch.int32).to(device), t.to(torch.int32).to(device)
 
 
 class Encoder(nn.Module):
@@ -401,10 +453,19 @@ class Encoder(nn.Module):
     def forward_ragged_packed(self, x, x_len, chunk=128):
         """forward_ragged for a CUDA batch sorted by decreasing length: the front end runs in ``chunk``-utterance
         pieces cropped to their own longest utterance, the valid frames are PACKED back to back and the
-        recurrent layers run over the packed frames (no padding is computed)."""
+        recurrent layers run over the packed frames (no padding is computed).  Sub-sampling layers keep the frames a
+        batch-1 call keeps (P, subsample_lengths) and the output holds rows [0, X) of each utterance, zeros beyond."""
         lens_host = x_len.cpu()
         n_utts = x.shape[0]
         front = self.layers[0] if isinstance(self.layers[0], VGGFrontEnd) else None
+        # P after every recurrent layer, from the host lengths: an utterance a layer would leave without frames is
+        # refused before anything is launched
+        p_host = x_host = lens_host.long().reshape(-1) // (4 if front is not None else 1)       # VGGFrontEnd: feat_len // 4
+        p_after = []
+        for layer in self.layers:
+            if isinstance(layer, RecurrentLayer):
+                p_host, x_host = subsample_lengths(p_host, x_host, layer.sample_rate, layer.sample_style)
+                p_after.append(p_host)
         packs, tls = [], []
         ready = getattr(self, "chunk_ready", None)      # decode_batch_from_host: rows [lo, hi) have arrived from the host
         for lo in range(0, n_utts, chunk):
@@ -430,13 +491,25 @@ class Encoder(nn.Module):
         first, rows = self._groups(t_host)
         g_first = torch.tensor(first, dtype=torch.int32, device=x.device)
         g_rows = torch.tensor(rows, dtype=torch.int32, device=x.device)
-        for layer in self.layers:
-            if isinstance(layer, RecurrentLayer):
-                feat = layer.forward_packed(feat, frame_off, lens32, g_first, g_rows)
-        t_max = int(t_host.max())
+        rec = [l for l in self.layers if isinstance(l, RecurrentLayer)]
+        for layer, p_out in zip(rec, p_after):
+            sub = layer.sample_rate > 1
+            feat = layer.forward_packed(feat, frame_off, lens32, g_first, g_rows, out_lens=p_out if sub else None)
+            if sub:
+                frame_off, lens32 = packed_offsets(p_out, x.device)
+                first, rows = self._groups(p_out)
+                g_first = torch.tensor(first, dtype=torch.int32, device=x.device)
+                g_rows = torch.tensor(rows, dtype=torch.int32, device=x.device)
+        enc_len, len_host = t_len, t_host
+        if any(l.sample_rate > 1 for l in rec):
+            enc_len, len_host = x_host.to(x.device), x_host
+            if not torch.equal(p_host, x_host):                           # keep rows [0, X) of each utterance's P
+                ar = torch.arange(int(p_host.max()), device=x.device)[None, :]
+                feat = feat[(ar < enc_len[:, None])[ar < p_host.to(x.device)[:, None]]]
+        t_max = int(len_host.max())
         enc = feat.new_zeros((n_utts, t_max, feat.shape[1]))
-        enc[torch.arange(t_max, device=x.device)[None, :] < t_len[:, None]] = feat
-        return enc, t_len
+        enc[torch.arange(t_max, device=x.device)[None, :] < enc_len[:, None]] = feat
+        return enc, enc_len
 
     def forward_ragged(self, x, x_len):
         """Batched encode of zero-padded utterances of different lengths with

@@ -520,6 +520,30 @@ def gru_sequence(gates, out, frame_off, lens, group_first, group_rows, hidden, f
                                      L.ptr(bw[0]), L.ptr(bw[1]), int(bw[2]), int(bw[3]), _stream()))
 
 
+def packed_subsample_ln(x, in_off, out_off, out_len, n_out, stride=1, g=1, weight=None, bias=None, eps=1e-5):
+    """LayerNorm and / or frame sub-sampling of packed utterances (see e2e_packed_subsample_ln): x [F, W] fp32 ->
+    out [n_out, g*W] with out[out_off[n] + j, s*W:(s+1)*W] = LN(x[in_off[n] + j*stride + s]) for j < out_len[n], s < g.
+    ``weight`` None: a plain gather.  n_out (a host int) is the number of output rows."""
+    _chk(x, F32, "x")
+    for t, nm in ((in_off, "in_off"), (out_off, "out_off"), (out_len, "out_len")):
+        _chk(t, I32, nm)
+    n = in_off.numel()
+    if x.dim() != 2 or out_off.numel() != n or out_len.numel() != n:
+        raise ValueError("packed_subsample_ln: x must be [F, W] and in_off / out_off / out_len of one length")
+    if weight is None and bias is not None:
+        raise ValueError("packed_subsample_ln: a LayerNorm bias needs its weight")
+    w = x.shape[1]
+    _chk(weight, F32, "weight", w)
+    _chk(bias, F32, "bias", w)
+    out = torch.empty((int(n_out), g * w), dtype=F32, device=x.device)
+    if n == 0 or n_out == 0:
+        return out
+    L.check(L.load().e2e_packed_subsample_ln(L.ptr(x), int(x.stride(0)), L.ptr(out), int(out.stride(0)), L.ptr(in_off),
+                                            L.ptr(out_off), L.ptr(out_len), int(n), int(w), int(stride), int(g),
+                                            L.ptr(weight), L.ptr(bias), float(eps), _stream()))
+    return out
+
+
 def conv1_direct(feat, weight, bias, valid_rows, n_freq, amax_out=None):
     """First VGG layer from the feature frames: feat [N,L,Cin*F] (last dim contiguous, rows of an utterance contiguous)
     -> relu(conv + bias) [N,L,F,Cout] NHWC.  ``amax_out`` (int32 [1], zeroed by the caller) receives the float bits of the

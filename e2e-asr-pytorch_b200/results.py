@@ -71,7 +71,9 @@ def decode_dataset(decoder, samples, device, max_utts=4096, max_padded_frames=0,
     feat_dim = int(samples[0][1].shape[1]) if len(samples) else 160
     bytes_fn = functools.partial(shard.estimate_decode_bytes, vocab=decoder.asr.vocab_size, beam=decoder.beam_size,
                                  n_cand=decoder.ctc_beam_size if decoder.apply_ctc else 0, feat_dim=feat_dim,
-                                 num_head=decoder.asr.attention.num_head, v_proj=bool(decoder.asr.attention.v_proj))
+                                 num_head=decoder.asr.attention.num_head, v_proj=bool(decoder.asr.attention.v_proj),
+                                 time_reduction=getattr(decoder.asr.encoder, "sample_rate", 4),
+                                 front_reduction=4 if getattr(decoder.asr.encoder, "vgg", 1) else 1)
     for batch in shard.make_batches(np.arange(len(samples)), lengths, max_utts, max_padded_frames, max_bytes, bytes_fn):
         l_max = int(lengths[batch].max())
         feats = torch.zeros(len(batch), l_max, samples[batch[0]][1].shape[1])

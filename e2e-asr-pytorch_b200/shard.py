@@ -42,7 +42,8 @@ def plan_shards(lengths, world_size, max_len_ratio=0.2):
 
 
 def estimate_decode_bytes(n_utts, l_max, vocab, beam, n_cand, feat_dim=160, enc_dim=640, att_dim=300,
-                          lm_dim=1024, lm_layers=4, encoder_chunk=128, num_head=1, v_proj=False):
+                          lm_dim=1024, lm_layers=4, encoder_chunk=128, num_head=1, v_proj=False, time_reduction=4,
+                          front_reduction=4):
     """Upper estimate of the HBM ``BeamDecoder.decode_batch`` needs at its peak for ``n_utts`` utterances padded
     to ``l_max`` input frames (DESIGN.md §3: every buffer is sized by the LONGEST utterance of the batch).
     Dominant terms: the frame-major posteriors together with the CTC logits they are made from
@@ -50,8 +51,14 @@ def estimate_decode_bytes(n_utts, l_max, vocab, beam, n_cand, feat_dim=160, enc_
     buffers, the encoder output and the attention keys; the encoder's chunk temporaries are a constant.  With
     ``num_head`` heads the keys and alignments are H times as large, and with ``v_proj`` the projected values
     [U][T][H*enc_dim] are held as well (~22 GB for 2620 utterances of ~828 frames at H = 4), counted twice because the
-    plain multi-head step holds a head-major copy beside them while it makes it."""
-    u, t = int(n_utts), (int(l_max) // 4 + 3) // 4 * 4
+    plain multi-head step holds a head-major copy beside them while it makes it.  ``time_reduction`` is the encoder's
+    input-to-output frame ratio (``Encoder.sample_rate``: 4 for the VGG front end alone, 2 for config/librispeech_asr.yaml's
+    encoder without it), ``front_reduction`` the part of it before the first recurrent layer (4 with the VGG front end, 1
+    without).  Where a recurrent layer sub-samples (the two differ) the terms at the output frame rate under-count the
+    encoder: its first recurrent layer runs over all U * l_max / front_reduction frames of the batch at once
+    (Encoder.forward_ragged_packed) and holds the packed input, the gates [F, 4*enc_dim], the recurrence output and the
+    sub-sampled output together; that term is added."""
+    u, t = int(n_utts), (int(l_max) // int(time_reduction) + 3) // 4 * 4
     vp = (int(vocab) + 3) // 4 * 4
     n = u * beam
     feats = u * int(l_max) * feat_dim * 4
@@ -66,7 +73,12 @@ def estimate_decode_bytes(n_utts, l_max, vocab, beam, n_cand, feat_dim=160, enc_
     lstm = n * (lm_layers * (3 * 2 * lm_dim * 2 + 4 * lm_dim * 4) + 4 * lm_dim * 4) + 3 * n * vp * 4
     hist = 3 * (int(l_max) // 5 + 2) * n * 4
     chunk = min(u, encoder_chunk) * int(l_max) * 40 * 128 * 4 * 3 + (3 << 30) * 2      # VGG activations + unfolded operand + GEMM result
-    return int(1.1 * (feats + enc + keys + values + post + states + attn + lstm + hist + chunk))
+    first = 0
+    if int(time_reduction) != int(front_reduction):
+        f1 = u * (int(l_max) // int(front_reduction))
+        in_w = feat_dim if int(front_reduction) == 1 else 4 * enc_dim    # the VGG output: 256 channels x F/4 bins (2560 at full size)
+        first = f1 * (in_w + 4 * enc_dim + 2 * enc_dim) * 4
+    return int(1.1 * (feats + enc + keys + values + post + states + attn + lstm + hist + chunk + first))
 
 
 def make_batches(indices, lengths, max_utts=512, max_padded_frames=None, max_bytes=None, bytes_fn=None):

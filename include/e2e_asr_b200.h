@@ -375,6 +375,19 @@ int e2e_gru_sequence(const float *gates, long long gates_pitch, float *out, long
                      const float *bias_bw, const float *w_t_bw, int gate_off_bw, int out_off_bw,
                      void *stream);
 
+/* What RNNLayer does to a layer's output between the recurrence and the projection (src/module.py:1003-1081:
+ * LayerNorm over the full output row, then sub-sampling by 'drop' or 'concat'), on packed utterances (csrc/encoder_post.cu):
+ *   out[out_off[n] + j][s*W : (s+1)*W] = LN(in[in_off[n] + j*stride + s])      for every n < N, j < out_len[n], s < g
+ *   LN(x) = (x - mean(x)) / sqrt(var(x) + eps) * ln_weight + ln_bias, mean and biased variance over the W values of the
+ *   row in fp32 (two passes, as nn.LayerNorm); ln_weight == NULL: no LayerNorm (a plain gather); ln_bias may be NULL.
+ * 'drop' by r: stride r, g = 1 (out_len = ceil(len / r));  'concat' by r: stride r, g = r (out_len = len / r, the len % r
+ * trailing frames are dropped);  LayerNorm alone: stride 1, g = 1.  g must be 1 or stride.  in_off / out_off / out_len
+ * are int32 device arrays [N]; the caller guarantees that every source row exists.  in_pitch >= W, out_pitch >= g*W
+ * (floats); out must not overlap in. */
+int e2e_packed_subsample_ln(const float *in, long long in_pitch, float *out, long long out_pitch,
+                            const int *in_off, const int *out_off, const int *out_len, int N, int W,
+                            int stride, int g, const float *ln_weight, const float *ln_bias, float eps, void *stream);
+
 /* First VGG layer (Conv2d Cin->Cout 3x3 "same" + bias + ReLU, src/module.py:672-674) straight from the feature
  * frames: feat [N][L][Cin*F] (a frame is Cin blocks of F bins, src/module.py:688-690; row pitch of an utterance
  * feat_pitch_n floats), weight [Cout][Cin][3][3], out [N][L][F][Cout] NHWC.  Input rows t >= valid_rows[n] read as 0. */
