@@ -46,6 +46,8 @@ SIGNATURES = {
                                     c_void_p, c_void_p, c_int, c_int, c_int,
                                     c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     "e2e_beam_candidates": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "e2e_emb_fuse_candidates": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int,
+                                        c_void_p, c_int, c_float, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "e2e_beam_combine_prune": (c_int, [c_void_p, c_int, c_void_p,
                                        c_void_p, c_int,
                                        c_void_p, c_void_p,

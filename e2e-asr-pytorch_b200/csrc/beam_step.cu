@@ -158,6 +158,115 @@ beam_candidates_kernel(const float *__restrict__ att_logits, int ld, int U, int 
 }
 
 // ---------------------------------------------------------------------------------------------
+// (3a') embedding fusion: (3a) for models decoded with the word-embedding plug-in (src/plugin.py,
+//       EmbeddingRegularizer.fuse_prob, called at src/decode.py:~118-122).  One warp per hypothesis.
+// ---------------------------------------------------------------------------------------------
+struct EmbFuseParams {
+    const float *dec; int ld_dec; const float *emb; int ld_emb;
+    int U, B, V, C;
+    const float *scale; int n_scale;        // relu(temp): 1 or V entries
+    const float *lam; int n_lam;            // the mixing weight (after the sigmoid of a learnable one): 1 or V entries
+    float eps;
+    const int *n_live; float *logp; int ld_out; float2 *att_stats; int *cand;
+};
+
+// log((1 - lam) * dec_prob + lam * emb_prob + eps), every operation rounded in plugin.py's order
+__device__ __forceinline__ float fused_logp(float pd, float pe, float lam, float eps)
+{
+    const float mix = __fadd_rn(__fmul_rn(__fsub_rn(1.0f, lam), pd), __fmul_rn(lam, pe));
+    return logf(__fadd_rn(mix, eps));
+}
+
+// softmax(x)[v] = exp(x[v] - max) * (1 / sum): the reciprocal form of ATen's row softmax
+template <int NV>
+__global__ void __launch_bounds__(kCandWarps * 32)
+emb_fuse_candidates_kernel(const EmbFuseParams p)
+{
+    const int lane = threadIdx.x & 31;
+    const int n = blockIdx.x * kCandWarps + (threadIdx.x >> 5);
+    if (n >= p.U * p.B) return;
+    const int u = n / p.B, b = n - u * p.B;
+    if (p.n_live && b >= p.n_live[u]) return;
+    const int V = p.V, C = p.C;
+    const float *drow = p.dec + (long long)n * p.ld_dec;
+    const float *erow = p.emb + (long long)n * p.ld_emb;
+    float *out = p.logp + (long long)n * p.ld_out;
+    auto scaled_emb = [&](int v) { return __fmul_rn(__ldg(p.scale + (p.n_scale == 1 ? 0 : v)), __ldg(erow + v)); };
+    auto lam_of = [&](int v) { return __ldg(p.lam + (p.n_lam == 1 ? 0 : v)); };
+    // (3b) forms its attention log-prob as (x - max) - lse: zero statistics pass the fused row through unchanged
+    if (lane == 0) p.att_stats[n] = make_float2(0.0f, 0.0f);
+    int *cand = C > 0 ? p.cand + (long long)n * C : nullptr;
+    auto emit = [&](int r, float, int idx) { if (lane == 0) cand[r] = idx; };
+    if constexpr (NV > 0) {
+        // narrow rows: both rows live in registers, one read of each
+        float xd[NV], xe[NV];
+        float md = -INFINITY, me = -INFINITY;
+#pragma unroll
+        for (int q = 0; q < NV; ++q) {
+            const int v = lane + 32 * q;
+            xd[q] = v < V ? __ldg(drow + v) : -INFINITY;
+            xe[q] = v < V ? scaled_emb(v) : -INFINITY;
+            md = fmaxf(md, xd[q]);
+            me = fmaxf(me, xe[q]);
+        }
+        md = warp_max(md);
+        me = warp_max(me);
+        float sd = 0.0f, se = 0.0f;
+#pragma unroll
+        for (int q = 0; q < NV; ++q) {
+            if (lane + 32 * q < V) {
+                xd[q] = expf(xd[q] - md);
+                xe[q] = expf(xe[q] - me);
+                sd += xd[q];
+                se += xe[q];
+            }
+        }
+        const float rd = __fdiv_rn(1.0f, warp_sum(sd)), re = __fdiv_rn(1.0f, warp_sum(se));
+        float lp[NV];
+#pragma unroll
+        for (int q = 0; q < NV; ++q) {
+            const int v = lane + 32 * q;
+            lp[q] = -INFINITY;
+            if (v < V) {
+                lp[q] = fused_logp(__fmul_rn(xd[q], rd), __fmul_rn(xe[q], re), lam_of(v), p.eps);
+                out[v] = lp[q];
+            }
+        }
+        if (C > 0) warp_select_topk_cached<NV>(lp, V, C, lane, emit);
+    } else {
+        // wide rows: maxima, then sums, then one pass that writes the fused row and feeds the streaming top-C lists
+        float md = -INFINITY, me = -INFINITY;
+        for (int v = lane; v < V; v += 32) {
+            md = fmaxf(md, __ldg(drow + v));
+            me = fmaxf(me, scaled_emb(v));
+        }
+        md = warp_max(md);
+        me = warp_max(me);
+        float sd = 0.0f, se = 0.0f;
+        for (int v = lane; v < V; v += 32) {
+            sd += expf(__ldg(drow + v) - md);
+            se += expf(scaled_emb(v) - me);
+        }
+        const float rd = __fdiv_rn(1.0f, warp_sum(sd)), re = __fdiv_rn(1.0f, warp_sum(se));
+        auto visit = [&](int v) -> float {
+            const float pd = __fmul_rn(expf(__ldg(drow + v) - md), rd);
+            const float pe = __fmul_rn(expf(scaled_emb(v) - me), re);
+            const float lp = fused_logp(pd, pe, lam_of(v), p.eps);
+            out[v] = lp;
+            return lp;
+        };
+        if (C > 0) {
+            extern __shared__ __align__(16) unsigned char fuse_smem[];           // [warps][C][32] values | [warps][C][32] ids
+            float *lv = reinterpret_cast<float *>(fuse_smem) + (size_t)(threadIdx.x >> 5) * C * 32;
+            int *li = reinterpret_cast<int *>(fuse_smem) + (size_t)kCandWarps * C * 32 + (size_t)(threadIdx.x >> 5) * C * 32;
+            warp_select_topk_stream(V, C, lane, visit, emit, lv, li);
+        } else {
+            for (int v = lane; v < V; v += 32) visit(v);
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
 // (3b) one CTA per utterance, one warp per parent hypothesis, then a pooled rank sort
 // ---------------------------------------------------------------------------------------------
 struct CombineParams {
@@ -580,6 +689,38 @@ extern "C" int e2e_beam_candidates(const float *att_logits, int ld, int U, int B
         att_logits, ld, U, B, V, C, n_live, reinterpret_cast<float2 *>(att_stats), cand);
     count_launch();
     return check_launch("e2e_beam_candidates");
+}
+
+extern "C" int e2e_emb_fuse_candidates(const float *dec_logits, int ld_dec, const float *emb_logits, int ld_emb,
+                                       int U, int B, int V, int C, const float *scale, int n_scale,
+                                       const float *lam, int n_lam, float eps, const int *n_live,
+                                       float *logp, int ld_out, float *att_stats, int *cand, void *stream)
+{
+    using namespace e2e;
+    if (!dec_logits || !emb_logits || !scale || !lam || !logp || !att_stats || (C > 0 && !cand))
+        return set_error(E2E_ERR_ARG, "e2e_emb_fuse_candidates: null pointer");
+    if (U <= 0 || B <= 0 || V <= 0 || C < 0 || C > V || ld_dec < V || ld_emb < V || ld_out < V)
+        return set_error(E2E_ERR_ARG, "e2e_emb_fuse_candidates: bad size");
+    if ((n_scale != 1 && n_scale != V) || (n_lam != 1 && n_lam != V))
+        return set_error(E2E_ERR_ARG, "e2e_emb_fuse_candidates: scale / lam must have 1 or V entries");
+    if (!(eps > 0.0f) || !isfinite(eps)) return set_error(E2E_ERR_ARG, "e2e_emb_fuse_candidates: eps must be positive and finite");
+    EmbFuseParams p;
+    p.dec = dec_logits; p.ld_dec = ld_dec; p.emb = emb_logits; p.ld_emb = ld_emb;
+    p.U = U; p.B = B; p.V = V; p.C = C;
+    p.scale = scale; p.n_scale = n_scale; p.lam = lam; p.n_lam = n_lam; p.eps = eps;
+    p.n_live = n_live; p.logp = logp; p.ld_out = ld_out; p.att_stats = reinterpret_cast<float2 *>(att_stats); p.cand = cand;
+    const int N = U * B;
+    void (*kern)(EmbFuseParams) = V <= 32 ? emb_fuse_candidates_kernel<1> : V <= 64 ? emb_fuse_candidates_kernel<2>
+                                : V <= 128 ? emb_fuse_candidates_kernel<4> : emb_fuse_candidates_kernel<0>;
+    const size_t smem = V > 128 ? (size_t)kCandWarps * C * 32 * 8 : 0;      // per-lane top-C lists of the streaming selection
+    if (smem > 48 * 1024) {
+        if (smem > 200 * 1024) return set_error(E2E_ERR_UNSUPPORTED, "e2e_emb_fuse_candidates: C too large");
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return set_error(E2E_ERR_LAUNCH, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+    }
+    kern<<<(N + kCandWarps - 1) / kCandWarps, kCandWarps * 32, smem, static_cast<cudaStream_t>(stream)>>>(p);
+    count_launch();
+    return check_launch("e2e_emb_fuse_candidates");
 }
 
 extern "C" int e2e_beam_combine_prune(const float *att_logits, int ld_att, const float *att_stats,

@@ -8,7 +8,7 @@ Mirrors the interface of ``/root/reference/src/decode.py``:
 * ``.forward(audio_feature[1,L,D], feature_len[1]) -> list[Hypothesis]`` best first
   (decode.py:65-183), ``.create_msg()`` (decode.py:50-63) and the public attributes
   ``beam_size, min_len_ratio, max_len_ratio, asr, apply_ctc, ctc_w, ctc_beam_size,
-  apply_lm, lm_w, lm_path, lm, apply_emb``
+  apply_lm, lm_w, lm_path, lm, apply_emb, emb_decoder``
 * ``Hypothesis.outIndex`` / ``.avgScore()`` / ``.output_seq`` / ``.output_scores``
   (decode.py:186-217,279-281)
 
@@ -18,7 +18,8 @@ the reference fans single utterances out to joblib processes
 (``bin/test_asr.py:138-139``); here they share every kernel launch.
 
 Per decode step the device runs: the batched PyTorch model step (``stepper.py``),
-then (3a) ``e2e_beam_candidates``, (2) ``e2e_ctc_prefix_step`` (the fused lazy prefix
+then (3a) ``e2e_beam_candidates`` (``e2e_emb_fuse_candidates`` for a model decoded with the word-embedding
+fusion plug-in, ``emb_decoder``), (2) ``e2e_ctc_prefix_step`` (the fused lazy prefix
 kernel; ``e2e_ctc_prefix_score``, the eager one, with ``lazy_prefix = False``), (3b)
 ``e2e_beam_combine_prune``; the posteriors come from (1) ``e2e_ctc_log_softmax``
 once per batch.  Nothing is copied to the host until the final N-best.
@@ -120,7 +121,13 @@ class BeamDecoder(nn.Module):
 
         self.apply_emb = emb_decoder is not None
         if self.apply_emb:
-            raise NotImplementedError("embedding-fusion decoding (src/plugin.py) is outside the decode hot-path scope")
+            # the word-embedding fusion plug-in (src/plugin.py EmbeddingRegularizer, model.EmbeddingRegularizer)
+            if getattr(emb_decoder, "use_bert", False):
+                raise NotImplementedError("embedding fusion with a BERT table (use_bert) is not supported")
+            if not getattr(emb_decoder, "apply_fuse", False):
+                # the reference would take the plug-in's None log-prob as the attention scores and fail on it
+                raise ValueError("emb_decoder has no probability fusion (apply_fuse is False, fuse == 0): nothing to decode with")
+            self.emb_decoder = emb_decoder
 
         # knobs of the device path (not part of the reference interface)
         self.fast_math = False          # MUFU log-add-exp in the prefix-score kernel
@@ -168,6 +175,9 @@ class BeamDecoder(nn.Module):
             msg.append('           |Joint CTC decoding enabled \t| weight = {:.2f}\t'.format(self.ctc_w))
         if self.apply_lm:
             msg.append('           |Joint LM decoding enabled \t| weight = {:.2f}\t| src = {}'.format(self.lm_w, self.lm_path))
+        if self.apply_emb:
+            msg.append('           |Joint Emb. decoding enabled \t| weight = {:.2f}'.format(
+                float(self.emb_decoder.fuse_lambda.mean().cpu().item())))
         return msg
 
     # ------------------------------------------------------------------------------------------
@@ -305,11 +315,12 @@ class BeamDecoder(nn.Module):
 
         with _Fp32Math():
             mark("start", True)
-            knobs = (self.split_gemm, self.fused_attention, self.lm_split, self.vgg_split, self.step_graphs, self.vgg_conv)
+            emb = self.emb_decoder if self.apply_emb else None
+            knobs = (self.split_gemm, self.fused_attention, self.lm_split, self.vgg_split, self.step_graphs, self.vgg_conv, emb)
             if self._stepper is None or self._stepper[0] != dev or self._stepper[1] != knobs:
                 self._stepper = (dev, knobs, BatchedStepper(self.asr, self.lm if self.apply_lm else None,
                                                             self.split_gemm, self.fused_attention, self.lm_split, self.vgg_split,
-                                                            self.step_graphs, self.vgg_conv))
+                                                            self.step_graphs, self.vgg_conv, emb))
             stepper = self._stepper[2]
             stepper.mark = mark
             enc, enc_len = stepper.encode(audio_feature, feature_len.to(dev))
@@ -318,6 +329,9 @@ class BeamDecoder(nn.Module):
             stepper.start(enc, enc_len, beam)
             t_max = enc.shape[1]
             buf = ops.BeamBuffers(n_utts, beam, n_cand, n_steps, min_len, max_len, dev)
+            fusion = stepper.emb
+            if fusion is not None:
+                fused = torch.empty((n_utts * beam, vocab), dtype=torch.float32, device=dev)     # the fused log-probs of a step
             r_prev = r_a = r_b = x = None
             if self.apply_ctc:
                 lin = self.asr.ctc_layer[0]
@@ -337,9 +351,16 @@ class BeamDecoder(nn.Module):
             mark("ctc_posterior", True)
             for step in range(n_steps):                                            # decode.py:104
                 k = n_run[step]
-                att_logits, lm_logits = stepper.step(buf.last_tok64[:k].view(-1), k)
-                mark("step_rest")
-                ops.beam_candidates(att_logits, k, beam, vocab, n_cand, buf.n_active, buf.att_stats, buf.cand)
+                if fusion is None:
+                    att_logits, lm_logits = stepper.step(buf.last_tok64[:k].view(-1), k)
+                    mark("step_rest")
+                    ops.beam_candidates(att_logits, k, beam, vocab, n_cand, buf.n_active, buf.att_stats, buf.cand)
+                else:
+                    # embedding fusion: the fused log-probs take the attention log-softmax's place, with zero statistics
+                    dec_logits, lm_logits, emb_logits = stepper.step(buf.last_tok64[:k].view(-1), k)
+                    mark("step_rest")
+                    att_logits = ops.emb_fuse_candidates(dec_logits, emb_logits, k, beam, vocab, n_cand, fusion.scale, fusion.lam,
+                                                         fusion.eps, buf.n_active, fused[:k * beam], buf.att_stats, buf.cand)
                 if self.apply_ctc:
                     r_cur = r_a if (step % 2 == 0) else r_b
                     if self.profile_prefix:

@@ -25,7 +25,8 @@ its own batched step.
 Supported subset (what the shipped configs under ``config/`` need for decode):
 encoder ``vgg`` 0/1 + (B)LSTM/GRU layers with drop/concat sub-sampling, optional
 LayerNorm and projection; attention ``loc`` or ``dot``; LSTM/GRU decoder; RNNLM
-LSTM/GRU with or without embedding tying.
+LSTM/GRU with or without embedding tying; the decode-time probability fusion of the
+word-embedding plug-in (``EmbeddingRegularizer``, ``src/plugin.py``).
 """
 import math
 
@@ -738,3 +739,74 @@ class RNNLM(nn.Module):
         out, _ = nn.utils.rnn.pad_packed_sequence(out, batch_first=True)
         out = F.linear(self.dp2(out), self.emb.weight) if self.emb_tying else self.trans(self.dp2(out))
         return out, hidden
+
+
+class EmbeddingRegularizer(nn.Module):
+    """The decode subset of the word-embedding plug-in (src/plugin.py EmbeddingRegularizer), with its parameter and
+    buffer names and shapes, so that ``load_state_dict`` works both ways: ``emb_table.weight`` [V, E],
+    ``emb_net.{0,2}.{weight,bias}`` (Linear(D, (D+E)//2) -> ReLU -> Linear((D+E)//2, E)), ``fuse_lambda`` and ``temp``.
+
+    ``fuse``: a fixed mixing weight in (0, 1] (buffer [1]), -1 (learnable scalar, parameter [1], used through a sigmoid)
+    or -2 (learnable per vocabulary entry, parameter [V]); 0 switches the fusion off (``apply_fuse`` False).
+    ``temperature``: fixed (buffer [1]), -1 (learnable scalar) or -2 (learnable per entry, [V]); used as relu(temp).
+    The table comes as a tensor ``table`` [V, E] or, with ``emb_dim``, as a random N(0, 1) one of that width (load a
+    checkpoint over it).  The BERT table and the training-time regulariser loss are not restated."""
+
+    def __init__(self, vocab_size, dec_dim, emb_dim=None, table=None, fuse=0.5, temperature=1.0, fuse_normalize=False,
+                 freeze=True):
+        super().__init__()
+        if table is None:
+            if emb_dim is None:
+                raise ValueError("EmbeddingRegularizer needs emb_dim or a table")
+            table = torch.randn(vocab_size, emb_dim)
+        table = torch.as_tensor(table, dtype=torch.float32)
+        if table.dim() != 2 or table.shape[0] != vocab_size:
+            raise ValueError("the embedding table must be [vocab_size, E]")
+        self.enable, self.use_bert, self.apply_dropout = True, False, False
+        self.emb_table = nn.Embedding.from_pretrained(table.clone(), freeze=freeze, padding_idx=0)
+        self.dim = self.emb_table.weight.shape[1]
+        self.emb_net = nn.Sequential(nn.Linear(dec_dim, (dec_dim + self.dim) // 2), nn.ReLU(),
+                                     nn.Linear((dec_dim + self.dim) // 2, self.dim))
+        self.fuse_normalize = fuse_normalize
+        self.apply_fuse = fuse != 0
+        if self.apply_fuse:
+            if fuse == -1:
+                self.fuse_type, self.fuse_learnable = "learnable", True
+                self.fuse_lambda = nn.Parameter(torch.FloatTensor([0.5]))
+            elif fuse == -2:
+                self.fuse_type, self.fuse_learnable = "vocab-wise learnable", True
+                self.fuse_lambda = nn.Parameter(torch.ones(vocab_size) * 0.5)
+            else:
+                self.fuse_type, self.fuse_learnable = str(fuse), False
+                self.register_buffer("fuse_lambda", torch.FloatTensor([fuse]))
+            if temperature == -1:
+                self.temperature = "learnable"
+                self.temp = nn.Parameter(torch.FloatTensor([1]))
+            elif temperature == -2:
+                self.temperature = "elementwise"
+                self.temp = nn.Parameter(torch.ones(vocab_size))
+            else:
+                self.temperature = str(temperature)
+                self.register_buffer("temp", torch.FloatTensor([temperature]))
+            self.eps = 1e-8
+
+    def fuse_prob(self, x_emb, dec_logit):
+        """log((1 - lam) * softmax(dec_logit) + lam * softmax(relu(temp) * emb_logit) + eps)."""
+        if self.fuse_normalize:
+            emb_logit = F.linear(F.normalize(x_emb, dim=-1), F.normalize(self.emb_table.weight, dim=-1))
+        else:
+            emb_logit = F.linear(x_emb, self.emb_table.weight)
+        emb_prob = (F.relu(self.temp) * emb_logit).softmax(dim=-1)
+        dec_prob = dec_logit.softmax(dim=-1)
+        if self.fuse_learnable:
+            fused_prob = (1 - torch.sigmoid(self.fuse_lambda)) * dec_prob + torch.sigmoid(self.fuse_lambda) * emb_prob
+        else:
+            fused_prob = (1 - self.fuse_lambda) * dec_prob + self.fuse_lambda * emb_prob
+        return (fused_prob + self.eps).log()
+
+    def forward(self, dec_state, dec_logit, label=None, return_loss=False):
+        """(None, log_fused) as the plug-in returns with return_loss=False; log_fused is None without fusion."""
+        if return_loss:
+            raise NotImplementedError("the training-time embedding regulariser loss is outside the decode scope")
+        x_emb = self.emb_net(dec_state)
+        return None, (self.fuse_prob(x_emb, dec_logit) if self.apply_fuse else None)

@@ -132,6 +132,27 @@ def beam_candidates(att_logits, n_utts, beam, vocab, n_cand, n_live, att_stats, 
                                         L.ptr(n_live), L.ptr(att_stats), L.ptr(cand), _stream()))
 
 
+def emb_fuse_candidates(dec_logits, emb_logits, n_utts, beam, vocab, n_cand, scale, lam, eps, n_live, logp, att_stats, cand):
+    """beam_candidates for a model decoded with embedding fusion (see e2e_emb_fuse_candidates): the first n_utts*beam
+    rows of dec_logits / emb_logits [>=n_utts*beam, V] -> logp (the fused log-probs, rows of the same shape), zero
+    att_stats and the top-n_cand ids of logp.  scale = relu(temp) and lam (after the sigmoid of a learnable weight)
+    hold 1 or V entries."""
+    for t, nm in ((dec_logits, "dec_logits"), (emb_logits, "emb_logits"), (logp, "logp")):
+        _chk(t, F32, nm)
+        if t.dim() != 2 or t.shape[0] < n_utts * beam or t.shape[1] < vocab:
+            raise ValueError("%s must be [>=%d, >=%d]" % (nm, n_utts * beam, vocab))
+    _chk(scale, F32, "scale")
+    _chk(lam, F32, "lam")
+    _chk(n_live, I32, "n_live", n_utts)
+    _chk(att_stats, F32, "att_stats", n_utts * beam * 2)
+    _chk(cand, I32, "cand", n_utts * beam * n_cand)
+    L.check(L.load().e2e_emb_fuse_candidates(L.ptr(dec_logits), int(dec_logits.stride(0)), L.ptr(emb_logits), int(emb_logits.stride(0)),
+                                            int(n_utts), int(beam), int(vocab), int(n_cand), L.ptr(scale), int(scale.numel()),
+                                            L.ptr(lam), int(lam.numel()), float(eps), L.ptr(n_live), L.ptr(logp), int(logp.stride(0)),
+                                            L.ptr(att_stats), L.ptr(cand), _stream()))
+    return logp
+
+
 class BeamBuffers:
     """Device-resident beam-search bookkeeping for a batch of U utterances
     (the arrays e2e_beam_combine_prune updates in place)."""

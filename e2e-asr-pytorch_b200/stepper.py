@@ -369,10 +369,41 @@ class _FusedLstm:
         self.idx = idx
 
 
+class EmbFusion:
+    """The per-step operands of the word-embedding fusion plug-in (src/plugin.py EmbeddingRegularizer), read from the
+    module by the reference's parameter names, so the reference's own object works as well as model.py's.  What does
+    not change during a decode is prepared once: the row-normalised table (``fuse_normalize``), ``scale`` = relu(temp)
+    and ``lam``, the mixing weight (sigmoid of a learnable one).  :meth:`logits` is x_emb @ table^T of the speller's
+    top-layer output: two library GEMMs and a ReLU for emb_net, then the table product (fp32: the decode loop runs under
+    decode._Fp32Math)."""
+
+    def __init__(self, emb):
+        with torch.no_grad():
+            lin0, lin2 = emb.emb_net[0], emb.emb_net[2]
+            self.w0, self.b0 = lin0.weight.detach(), lin0.bias.detach()
+            self.w2, self.b2 = lin2.weight.detach(), lin2.bias.detach()
+            table = emb.emb_table.weight.detach()
+            self.normalize = bool(emb.fuse_normalize)
+            self.table = (F.normalize(table, dim=-1) if self.normalize else table).contiguous()
+            self.scale = F.relu(emb.temp.detach()).float().contiguous()
+            lam = emb.fuse_lambda.detach()
+            self.lam = (torch.sigmoid(lam) if emb.fuse_learnable else lam).float().contiguous()
+            self.eps = float(emb.eps)
+
+    def logits(self, top):
+        """top [n, D] -> emb_logits [n, V]."""
+        x = F.linear(F.relu(F.linear(top, self.w0, self.b0)), self.w2, self.b2)
+        if self.normalize:
+            x = F.normalize(x, dim=-1)
+        return F.linear(x, self.table)
+
+
 class BatchedStepper:
     def __init__(self, asr, lm=None, split_gemm=False, fused_attention=False, lm_split="bf16x3", vgg_split="bf16x3", step_graphs=False,
-                 vgg_conv="igemm"):
+                 vgg_conv="igemm", emb=None):
         att = asr.attention
+        # the word-embedding fusion plug-in (None: off); step() then also returns its logits
+        self.emb = EmbFusion(emb) if emb is not None else None
         if att.mode not in ("loc", "dot"):
             raise NotImplementedError("attention mode " + str(att.mode))
         self.asr, self.lm = asr, lm
@@ -585,8 +616,9 @@ class BatchedStepper:
     # -- once per decode step ---------------------------------------------------------------
     def step(self, prev_tok, k=None):
         """Advance the first ``k`` utterances (all by default).  prev_tok [k*B] long ->
-        (att_logits [k*B,V], lm_logits [k*B,V] | None); the new states are held until
-        :meth:`reorder` commits them in the surviving hypotheses' order."""
+        (att_logits [k*B,V], lm_logits [k*B,V] | None), and emb_logits [k*B,V] third when the stepper has an
+        embedding-fusion plug-in; the new states are held until :meth:`reorder` commits them in the surviving
+        hypotheses' order."""
         asr, att = self.asr, self.asr.attention
         k = self.U if k is None else k
         b, t = self.B, self.T
@@ -605,6 +637,7 @@ class BatchedStepper:
             dec_in = torch.cat([asr.pre_embed(prev_tok), context], dim=-1)
             top, self._new_dec = self.dec.step(dec_in, self.dec_state, n)
         att_logits = asr.decoder.char_trans(top)                                   # asr.py:265
+        emb_logits = self.emb.logits(top) if self.emb is not None else None       # plugin.py fuse_prob, from d_state = top
         self._new_att = (attn.view(n, t) if self.H == 1 else attn) if self.mode == "loc" else None
         self.mark("step_speller")
         lm_logits = None
@@ -616,7 +649,8 @@ class BatchedStepper:
                 top, self._new_lm = self.lm_rnn.step(x0, self.lm_state, n, tok=prev_tok)
             lm_logits = F.linear(top, self.lm.emb.weight) if self.lm.emb_tying else self.lm.trans(top)   # lm.py:33-37
             self.mark("step_lm")
-        return att_logits.contiguous(), (lm_logits.contiguous() if lm_logits is not None else None)
+        out = att_logits.contiguous(), (lm_logits.contiguous() if lm_logits is not None else None)
+        return out if emb_logits is None else out + (emb_logits.contiguous(),)
 
     def reorder(self, parent_row):
         """parent_row [U,B] int64 (row u*B + slot of each survivor's parent, written by e2e_beam_combine_prune):

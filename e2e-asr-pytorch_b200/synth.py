@@ -8,7 +8,7 @@ import copy
 import numpy as np
 import torch
 
-from .model import ASR, RNNLM
+from .model import ASR, RNNLM, EmbeddingRegularizer
 
 # Dimensions of config/librispeech_asr.yaml:42-68 with the VGG front end switched
 # on (vgg: 1, sample_rate [1,1,1,1] -> 4x time reduction), see SURVEY.md §8d.
@@ -62,6 +62,30 @@ def build_lm(vocab_size=31, cfg=None, seed=1, peak=1.0):
         with torch.no_grad():
             lm.emb.weight.mul_(peak)
     return lm
+
+
+def build_emb(vocab_size=31, dec_dim=300, emb_dim=300, fuse=0.5, temperature=1.0, fuse_normalize=False, seed=3,
+              perturb=True):
+    """Random-init embedding-fusion plug-in (model.EmbeddingRegularizer) in eval mode: an N(0, 1) table [V, E] and the
+    default Linear init of emb_net.  ``perturb`` moves the learnable weights away from their init values (seeded): a
+    learnable ``fuse_lambda`` to N(0, 1) logits, a learnable scalar ``temp`` to U(0.5, 2), an elementwise ``temp`` to
+    U(-0.5, 2) per entry with entry 2 set to -1, so that the ReLU clamps some of them to zero."""
+    g = torch.Generator().manual_seed(int(seed))
+    table = torch.randn(vocab_size, emb_dim, generator=g)
+    torch.manual_seed(seed)
+    emb = EmbeddingRegularizer(vocab_size, dec_dim, table=table, fuse=fuse, temperature=temperature,
+                               fuse_normalize=fuse_normalize).eval()
+    if perturb and emb.apply_fuse:
+        with torch.no_grad():
+            if emb.fuse_learnable:
+                emb.fuse_lambda.copy_(torch.randn(emb.fuse_lambda.shape, generator=g))
+            if temperature == -1:
+                emb.temp.copy_(0.5 + 1.5 * torch.rand(1, generator=g))
+            elif temperature == -2:
+                t = -0.5 + 2.5 * torch.rand(vocab_size, generator=g)
+                t[min(2, vocab_size - 1)] = -1.0
+                emb.temp.copy_(t)
+    return emb
 
 
 def utterance(i, n_frames, feat_dim=FEAT_DIM):

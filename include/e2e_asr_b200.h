@@ -148,6 +148,22 @@ int e2e_ctc_prefix_step(const float *x, int Tmax, int U, int Vp, int V, const in
 int e2e_beam_candidates(const float *att_logits, int ld, int U, int B, int V, int C,
                         const int *n_live, float *att_stats, int *cand, void *stream);
 
+/* (3a') (3a) for models decoded with the word-embedding fusion plug-in: replaces
+ * self.emb_decoder(d_state, cur_prob, return_loss=False) (src/decode.py:~118-122, src/plugin.py fuse_prob) and
+ * cur_prob.topk(ctc_beam_size).  Rows b >= n_live[u] of an utterance are not touched (n_live may be NULL).
+ *   dec_logits [U*B][ld_dec]  decoder outputs (char_trans), emb_logits [U*B][ld_emb] x_emb @ table^T (normalised
+ *                             operands with fuse_normalize), row pitches >= V
+ *   scale      [n_scale]      relu(temp), n_scale = 1 or V
+ *   lam        [n_lam]        the mixing weight (sigmoid(fuse_lambda) when learnable), n_lam = 1 or V
+ *   eps        > 0            added before the log (1e-8 in the plug-in)
+ *   logp       [U*B][ld_out]  out: log((1-lam)*softmax(dec) + lam*softmax(scale*emb) + eps), ld_out >= V
+ *   att_stats  [U*B][2]       out: (0, 0), so that (3b)'s (x - max) - lse reads logp unchanged
+ *   cand       [U*B][C]       out: ids of the C largest logp, best first (ties: lower id first); C may be 0 */
+int e2e_emb_fuse_candidates(const float *dec_logits, int ld_dec, const float *emb_logits, int ld_emb,
+                            int U, int B, int V, int C, const float *scale, int n_scale,
+                            const float *lam, int n_lam, float eps, const int *n_live,
+                            float *logp, int ld_out, float *att_stats, int *cand, void *stream);
+
 /* (3b) Score combine + <eos> threshold + top-k + length-normalised prune of one decode
  * step for every utterance.  Replaces src/decode.py:134-177 and Hypothesis.addTopk /
  * avgScore (src/decode.py:214-263).
