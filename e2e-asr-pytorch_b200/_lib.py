@@ -92,6 +92,12 @@ SIGNATURES = {
     "e2e_gru_sequence": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p, c_void_p,
                                  c_int, c_int, c_int, c_int,
                                  c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p]),
+    "e2e_lstm_sequence_wide": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p, c_void_p,
+                                       c_int, c_int, c_int, c_int,
+                                       c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p]),
+    "e2e_gru_sequence_wide": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p, c_void_p,
+                                      c_int, c_int, c_int, c_int,
+                                      c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "e2e_packed_subsample_ln": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p,
                                         c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_void_p]),
     "e2e_conv1_direct": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,

@@ -5,7 +5,7 @@
 //   out[out_off[n] + j][s*W : (s+1)*W] = LN(in[in_off[n] + j*stride + s])      for j < out_len[n], s < g
 // drop: stride r, g = 1;  concat: stride r, g = r;  LayerNorm alone: stride 1, g = 1.
 // One warp per source row: the mean, then the biased variance around it (two passes, as nn.LayerNorm), then the
-// normalised row.  The row (at most 2 x 384 floats) is read three times; the second and third reads hit L1.  Memory
+// normalised row.  The row (at most 2 x 1024 floats) is read three times; the second and third reads hit L1.  Memory
 // bound, no tensor cores.
 #include "common.cuh"
 

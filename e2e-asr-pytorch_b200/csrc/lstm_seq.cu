@@ -17,11 +17,21 @@
 // out [k][unit][4] = (W_hr, W_hz, W_hn, 0), so the recurrence keeps one 16-byte load per unit per k and runs 3R
 // accumulators (r, z and the n_h product, which starts at b_hn); the input half of the n gate is held apart (one value
 // per utterance) and the cell is ATen's order n = tanh(n_x + r * n_h), h' = (h - n) * u + n.
+//
+// Wider layers (lstm_seq_wide_kernel / gru_seq_wide_kernel, H a multiple of 128 up to 1024) run the same per-unit body
+// in a thread-block cluster of CL CTAs per (utterance group x direction): CTA c owns units [c H/CL, (c+1) H/CL), one
+// thread per unit as above, CL the smallest power of two >= 2 with H/CL <= 384.  Every CTA holds the FULL previous state
+// [2][H][R] in its shared memory; after its cell update a thread stores its R new values into the same slot of every
+// CTA of the cluster (mapa + st.shared::cluster), and one cluster barrier (arrive.release / wait.acquire) per time step
+// takes the place of the __syncthreads.  Gate loads, biases, the k = 0..H-1 FMA order and the cell are the narrow
+// kernel's, so for an H both accept the two give the same bits.
 #include "common.cuh"
 
 namespace e2e {
 
 constexpr int kSeqMaxThreads = 384;     // hidden sizes up to 384 (the register file then allows ~170 registers per thread)
+constexpr int kSeqWideMaxH = 1024;      // the cluster form: H % kSeqWideUnit == 0, H <= kSeqWideMaxH
+constexpr int kSeqWideUnit = 128;       // so that H / CL is whole warps for CL in {2, 4}
 
 struct SeqDir {
     const float *bias;      // [4H] b_ih + b_hh (may be null); GRU: [b_ir + b_hr | b_iz + b_hz | b_in | b_hn]
@@ -42,21 +52,54 @@ struct SeqParams {
 
 __device__ __forceinline__ float seq_sigmoid(float x) { return __fdiv_rn(1.0f, __fadd_rn(1.0f, expf(-x))); }
 
-template <bool kGru, int R>
+__device__ __forceinline__ unsigned cluster_ctarank()
+{
+    unsigned r;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+    return r;
+}
+
+__device__ __forceinline__ unsigned cluster_nctarank()
+{
+    unsigned r;
+    asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
+    return r;
+}
+
+// All threads of all CTAs of the cluster: shared-memory writes before it (local or remote) are visible after it.
+__device__ __forceinline__ void cluster_barrier()
+{
+    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+
+// 16-byte store to the same shared-memory offset as `local` in CTA `rank` of the cluster.
+__device__ __forceinline__ void st_cluster_f4(float *local, unsigned rank, float4 v)
+{
+    unsigned remote;
+    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"((unsigned)__cvta_generic_to_shared(local)), "r"(rank));
+    asm volatile("st.shared::cluster.v4.f32 [%0], {%1, %2, %3, %4};" :: "r"(remote), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
+}
+
+// kCluster: thread t of cluster CTA c owns unit c * blockDim.x + t and publishes its new state to every CTA's copy.
+// Otherwise thread u owns unit u of the CTA.
+template <bool kGru, int R, bool kCluster = false>
 __device__ __forceinline__ void lstm_seq_body(const SeqParams &p, const SeqDir &d, int first, int rows, float *smem)
 {
-    const int H = p.H, u = threadIdx.x;
+    const int H = p.H, t = threadIdx.x;
+    const int u = kCluster ? (int)cluster_ctarank() * blockDim.x + t : t;
     const bool unit = u < H;
     float *hs = smem;                                  // [2][H][R]
     int *s_len = reinterpret_cast<int *>(smem + 2 * H * R);
     int *s_off = s_len + R;
-    if (u < R) {
-        const bool ok = u < rows;
-        s_len[u] = ok ? p.lens[first + u] : 0;
-        s_off[u] = ok ? p.frame_off[first + u] : 0;
+    if (t < R) {
+        const bool ok = t < rows;
+        s_len[t] = ok ? p.lens[first + t] : 0;
+        s_off[t] = ok ? p.frame_off[first + t] : 0;
     }
-    for (int i = u; i < 2 * H * R; i += blockDim.x) hs[i] = 0.0f;
-    __syncthreads();
+    for (int i = t; i < 2 * H * R; i += blockDim.x) hs[i] = 0.0f;
+    // cluster: also no CTA writes into another's state before that one has started and zeroed it
+    if constexpr (kCluster) cluster_barrier();
+    else __syncthreads();
     int max_len = 0;
 #pragma unroll
     for (int r = 0; r < R; ++r) max_len = max(max_len, s_len[r]);
@@ -128,11 +171,26 @@ __device__ __forceinline__ void lstm_seq_body(const SeqParams &p, const SeqDir &
                     hout[r] = hc[u * R + r];                         // finished (or absent) utterance: state frozen
                 }
             }
+            if constexpr (kCluster) {
+                const unsigned n_cta = cluster_nctarank();
+                for (unsigned c = 0; c < n_cta; ++c)
 #pragma unroll
-            for (int q = 0; q < R / 4; ++q)
-                *reinterpret_cast<float4 *>(hn + u * R + 4 * q) = make_float4(hout[4 * q], hout[4 * q + 1], hout[4 * q + 2], hout[4 * q + 3]);
+                    for (int q = 0; q < R / 4; ++q)
+                        st_cluster_f4(hn + u * R + 4 * q, c, make_float4(hout[4 * q], hout[4 * q + 1], hout[4 * q + 2], hout[4 * q + 3]));
+            } else {
+#pragma unroll
+                for (int q = 0; q < R / 4; ++q)
+                    *reinterpret_cast<float4 *>(hn + u * R + 4 * q) = make_float4(hout[4 * q], hout[4 * q + 1], hout[4 * q + 2], hout[4 * q + 3]);
+            }
         }
-        __syncthreads();
+        // One barrier per step is enough because the state is double-buffered.  Step s reads buffer s & 1 and writes
+        // buffer (s + 1) & 1, in every CTA of the cluster.  After barrier s, every write of step s has been released
+        // and is acquired by all threads, so step s + 1 reads a complete state.  Step s + 1 then writes buffer s & 1,
+        // which step s read; a thread can only do that after passing barrier s, which every thread of every CTA reaches
+        // only after it has finished its step-s reads.  The last barrier also keeps each CTA (and its shared memory)
+        // alive until no other CTA of the cluster writes into it any more: all CTAs walk the same max_len steps.
+        if constexpr (kCluster) cluster_barrier();
+        else __syncthreads();
     }
 }
 
@@ -160,11 +218,27 @@ gru_seq_kernel(const SeqParams p)
     else lstm_seq_body<true, 16>(p, d, first, rows, seq_smem);
 }
 
+// Cluster form: grid (n_groups * CL, n_dirs), clusters of (CL, 1, 1), H / CL threads per CTA.
+template <bool kGru>
+__device__ __forceinline__ void seq_wide_run(const SeqParams &p)
+{
+    extern __shared__ __align__(16) float seq_smem[];
+    const int grp = blockIdx.x / cluster_nctarank();
+    const SeqDir &d = p.dir[blockIdx.y];
+    const int first = p.group_first[grp], rows = p.group_rows[grp];
+    if (rows <= 4) lstm_seq_body<kGru, 4, true>(p, d, first, rows, seq_smem);
+    else if (rows <= 8) lstm_seq_body<kGru, 8, true>(p, d, first, rows, seq_smem);
+    else lstm_seq_body<kGru, 16, true>(p, d, first, rows, seq_smem);
+}
+
+__global__ void __launch_bounds__(kSeqMaxThreads, 1) lstm_seq_wide_kernel(const SeqParams p) { seq_wide_run<false>(p); }
+__global__ void __launch_bounds__(kSeqMaxThreads, 1) gru_seq_wide_kernel(const SeqParams p) { seq_wide_run<true>(p); }
+
 }  // namespace e2e
 
 namespace {
 
-int sequence_impl(const char *name, bool gru, const float *gates, long long gates_pitch, float *out, long long out_pitch,
+int sequence_impl(const char *name, bool gru, bool wide, const float *gates, long long gates_pitch, float *out, long long out_pitch,
                   const int *frame_off, const int *lens, const int *group_first, const int *group_rows,
                   int N, int H, int n_groups, int n_dirs,
                   const float *bias_fw, const float *w_t_fw, int gate_off_fw, int out_off_fw,
@@ -176,48 +250,67 @@ int sequence_impl(const char *name, bool gru, const float *gates, long long gate
         return set_error(E2E_ERR_ARG, "%s: null pointer", name);
     if (N <= 0 || H <= 0 || n_groups <= 0 || (n_dirs != 1 && n_dirs != 2) || gates_pitch < (long long)n_gates * H || out_pitch < H)
         return set_error(E2E_ERR_ARG, "%s: bad size", name);
-    if (H > kSeqMaxThreads) return set_error(E2E_ERR_UNSUPPORTED, "%s: hidden size %d > %d", name, H, kSeqMaxThreads);
+    if (!wide && H > kSeqMaxThreads) return set_error(E2E_ERR_UNSUPPORTED, "%s: hidden size %d > %d", name, H, kSeqMaxThreads);
+    if (wide && (H % kSeqWideUnit || H > kSeqWideMaxH))
+        return set_error(E2E_ERR_UNSUPPORTED, "%s: hidden size %d is not a multiple of %d up to %d", name, H, kSeqWideUnit, kSeqWideMaxH);
     SeqParams p;
     p.gates = gates; p.gates_pitch = gates_pitch; p.out = out; p.out_pitch = out_pitch;
     p.frame_off = frame_off; p.lens = lens; p.group_first = group_first; p.group_rows = group_rows;
     p.N = N; p.H = H; p.n_groups = n_groups;
     p.dir[0] = SeqDir{bias_fw, w_t_fw, gate_off_fw, out_off_fw, 0};
     p.dir[1] = SeqDir{bias_bw, w_t_bw, gate_off_bw, out_off_bw, 1};
-    const int threads = (H + 31) / 32 * 32;
     const size_t smem = ((size_t)2 * H * 16 + 2 * 16) * 4;
     if (smem > 200 * 1024) return set_error(E2E_ERR_UNSUPPORTED, "%s: %zu bytes of shared memory needed", name, smem);
-    const auto kernel = gru ? gru_seq_kernel : lstm_seq_kernel;
+    const auto kernel = wide ? (gru ? gru_seq_wide_kernel : lstm_seq_wide_kernel) : (gru ? gru_seq_kernel : lstm_seq_kernel);
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return set_error(E2E_ERR_LAUNCH, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     }
-    kernel<<<dim3(n_groups, n_dirs), threads, smem, static_cast<cudaStream_t>(stream)>>>(p);
+    if (!wide) {
+        const int threads = (H + 31) / 32 * 32;
+        kernel<<<dim3(n_groups, n_dirs), threads, smem, static_cast<cudaStream_t>(stream)>>>(p);
+        count_launch();
+        return check_launch(name);
+    }
+    int cl = 2;                                         // the smallest power of two >= 2 with H / CL <= 384
+    while (H / cl > kSeqMaxThreads) cl *= 2;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = cl; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(n_groups * cl, n_dirs);
+    cfg.blockDim = dim3(H / cl);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = static_cast<cudaStream_t>(stream);
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    int clusters = 0;
+    cudaError_t e = cudaOccupancyMaxActiveClusters(&clusters, kernel, &cfg);
+    if (e != cudaSuccess) return set_error(E2E_ERR_LAUNCH, "%s: cudaOccupancyMaxActiveClusters: %s", name, cudaGetErrorString(e));
+    if (clusters <= 0)
+        return set_error(E2E_ERR_UNSUPPORTED, "%s: a cluster of %d CTAs x %d threads with %zu bytes of shared memory each does not fit",
+                         name, cl, H / cl, smem);
+    e = cudaLaunchKernelEx(&cfg, kernel, p);
+    if (e != cudaSuccess) return set_error(E2E_ERR_LAUNCH, "%s: cudaLaunchKernelEx: %s", name, cudaGetErrorString(e));
     count_launch();
     return check_launch(name);
 }
 
 }  // namespace
 
-extern "C" int e2e_lstm_sequence(const float *gates, long long gates_pitch, float *out, long long out_pitch,
-                                 const int *frame_off, const int *lens, const int *group_first, const int *group_rows,
-                                 int N, int H, int n_groups, int n_dirs,
-                                 const float *bias_fw, const float *w_t_fw, int gate_off_fw, int out_off_fw,
-                                 const float *bias_bw, const float *w_t_bw, int gate_off_bw, int out_off_bw,
-                                 void *stream)
-{
-    return sequence_impl("e2e_lstm_sequence", false, gates, gates_pitch, out, out_pitch, frame_off, lens, group_first, group_rows,
-                         N, H, n_groups, n_dirs, bias_fw, w_t_fw, gate_off_fw, out_off_fw, bias_bw, w_t_bw, gate_off_bw, out_off_bw,
-                         stream);
-}
+#define E2E_SEQUENCE_ENTRY(fn, gru, wide)                                                                                   \
+    extern "C" int fn(const float *gates, long long gates_pitch, float *out, long long out_pitch,                          \
+                      const int *frame_off, const int *lens, const int *group_first, const int *group_rows,                \
+                      int N, int H, int n_groups, int n_dirs,                                                              \
+                      const float *bias_fw, const float *w_t_fw, int gate_off_fw, int out_off_fw,                          \
+                      const float *bias_bw, const float *w_t_bw, int gate_off_bw, int out_off_bw, void *stream)            \
+    {                                                                                                                      \
+        return sequence_impl(#fn, gru, wide, gates, gates_pitch, out, out_pitch, frame_off, lens, group_first, group_rows, \
+                             N, H, n_groups, n_dirs, bias_fw, w_t_fw, gate_off_fw, out_off_fw,                             \
+                             bias_bw, w_t_bw, gate_off_bw, out_off_bw, stream);                                            \
+    }
 
-extern "C" int e2e_gru_sequence(const float *gates, long long gates_pitch, float *out, long long out_pitch,
-                                const int *frame_off, const int *lens, const int *group_first, const int *group_rows,
-                                int N, int H, int n_groups, int n_dirs,
-                                const float *bias_fw, const float *w_t_fw, int gate_off_fw, int out_off_fw,
-                                const float *bias_bw, const float *w_t_bw, int gate_off_bw, int out_off_bw,
-                                void *stream)
-{
-    return sequence_impl("e2e_gru_sequence", true, gates, gates_pitch, out, out_pitch, frame_off, lens, group_first, group_rows,
-                         N, H, n_groups, n_dirs, bias_fw, w_t_fw, gate_off_fw, out_off_fw, bias_bw, w_t_bw, gate_off_bw, out_off_bw,
-                         stream);
-}
+E2E_SEQUENCE_ENTRY(e2e_lstm_sequence, false, false)
+E2E_SEQUENCE_ENTRY(e2e_gru_sequence, true, false)
+E2E_SEQUENCE_ENTRY(e2e_lstm_sequence_wide, false, true)
+E2E_SEQUENCE_ENTRY(e2e_gru_sequence_wide, true, true)

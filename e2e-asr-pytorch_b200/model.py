@@ -308,8 +308,9 @@ class RecurrentLayer(nn.Module):
 
     # -- packed device path (CUDA only; SURVEY §8f row f-4) ----------------------------------------------
     def packed_supported(self):
+        from .ops import sequence_supported
         rnn = self.layer
-        return isinstance(rnn, (nn.LSTM, nn.GRU)) and rnn.num_layers == 1 and rnn.hidden_size <= 384
+        return isinstance(rnn, (nn.LSTM, nn.GRU)) and rnn.num_layers == 1 and sequence_supported(rnn.hidden_size)
 
     def _packed_weights(self):
         from .stepper import SplitLinear

@@ -501,9 +501,23 @@ def conv_bias_relu_mask(y_nhwc, bias, valid_rows, amax_in=None, inv_w_scale=None
                                                        L.ptr(amax_in), float(inv_w_scale), L.ptr(amax_out), _stream()))
 
 
+# Hidden sizes of the packed recurrence: e2e_lstm_sequence / e2e_gru_sequence run one CTA per utterance group with one
+# thread per unit up to SEQ_MAX_H; the *_wide entry points split the units of a group over a thread-block cluster and
+# take multiples of SEQ_WIDE_UNIT up to SEQ_WIDE_MAX_H.
+SEQ_MAX_H = 384
+SEQ_WIDE_UNIT = 128
+SEQ_WIDE_MAX_H = 1024
+
+
+def sequence_supported(hidden):
+    """True for the hidden sizes lstm_sequence / gru_sequence accept."""
+    h = int(hidden)
+    return 0 < h <= SEQ_MAX_H or (h % SEQ_WIDE_UNIT == 0 and h <= SEQ_WIDE_MAX_H)
+
+
 def lstm_sequence(gates, out, frame_off, lens, group_first, group_rows, hidden, fw, bw=None):
-    """Packed (B)LSTM recurrence (see e2e_lstm_sequence).  gates [F, >=4H*dirs] fp32, out [F, >=H*dirs];
-    fw / bw = (bias [4H] | None, w_t [H,H,4], gate_off, out_off)."""
+    """Packed (B)LSTM recurrence (see e2e_lstm_sequence; e2e_lstm_sequence_wide above SEQ_MAX_H units).  gates
+    [F, >=4H*dirs] fp32, out [F, >=H*dirs]; fw / bw = (bias [4H] | None, w_t [H,H,4], gate_off, out_off)."""
     _chk(gates, F32, "gates")
     _chk(out, F32, "out")
     for t, nm in ((frame_off, "frame_off"), (lens, "lens"), (group_first, "group_first"), (group_rows, "group_rows")):
@@ -514,16 +528,19 @@ def lstm_sequence(gates, out, frame_off, lens, group_first, group_rows, hidden, 
         _chk(w, F32, "w_t", 4 * hidden * hidden)
     if bw is None:
         bw = (None, None, 0, 0)
-    L.check(L.load().e2e_lstm_sequence(L.ptr(gates), int(gates.stride(0)), L.ptr(out), int(out.stride(0)),
-                                      L.ptr(frame_off), L.ptr(lens), L.ptr(group_first), L.ptr(group_rows),
-                                      int(lens.numel()), int(hidden), int(group_first.numel()), len(dirs),
-                                      L.ptr(fw[0]), L.ptr(fw[1]), int(fw[2]), int(fw[3]),
-                                      L.ptr(bw[0]), L.ptr(bw[1]), int(bw[2]), int(bw[3]), _stream()))
+    lib = L.load()
+    fn = lib.e2e_lstm_sequence if hidden <= SEQ_MAX_H else lib.e2e_lstm_sequence_wide
+    L.check(fn(L.ptr(gates), int(gates.stride(0)), L.ptr(out), int(out.stride(0)),
+               L.ptr(frame_off), L.ptr(lens), L.ptr(group_first), L.ptr(group_rows),
+               int(lens.numel()), int(hidden), int(group_first.numel()), len(dirs),
+               L.ptr(fw[0]), L.ptr(fw[1]), int(fw[2]), int(fw[3]),
+               L.ptr(bw[0]), L.ptr(bw[1]), int(bw[2]), int(bw[3]), _stream()))
 
 
 def gru_sequence(gates, out, frame_off, lens, group_first, group_rows, hidden, fw, bw=None):
-    """Packed (B)GRU recurrence (see e2e_gru_sequence).  gates [F, >=3H*dirs] fp32, out [F, >=H*dirs];
-    fw / bw = (bias [4H] = [b_ir+b_hr | b_iz+b_hz | b_in | b_hn] | None, w_t [H,H,4] (lane 3 zero), gate_off, out_off)."""
+    """Packed (B)GRU recurrence (see e2e_gru_sequence; e2e_gru_sequence_wide above SEQ_MAX_H units).  gates
+    [F, >=3H*dirs] fp32, out [F, >=H*dirs]; fw / bw = (bias [4H] = [b_ir+b_hr | b_iz+b_hz | b_in | b_hn] | None,
+    w_t [H,H,4] (lane 3 zero), gate_off, out_off)."""
     _chk(gates, F32, "gates")
     _chk(out, F32, "out")
     for t, nm in ((frame_off, "frame_off"), (lens, "lens"), (group_first, "group_first"), (group_rows, "group_rows")):
@@ -534,11 +551,13 @@ def gru_sequence(gates, out, frame_off, lens, group_first, group_rows, hidden, f
         _chk(w, F32, "w_t", 4 * hidden * hidden)
     if bw is None:
         bw = (None, None, 0, 0)
-    L.check(L.load().e2e_gru_sequence(L.ptr(gates), int(gates.stride(0)), L.ptr(out), int(out.stride(0)),
-                                     L.ptr(frame_off), L.ptr(lens), L.ptr(group_first), L.ptr(group_rows),
-                                     int(lens.numel()), int(hidden), int(group_first.numel()), len(dirs),
-                                     L.ptr(fw[0]), L.ptr(fw[1]), int(fw[2]), int(fw[3]),
-                                     L.ptr(bw[0]), L.ptr(bw[1]), int(bw[2]), int(bw[3]), _stream()))
+    lib = L.load()
+    fn = lib.e2e_gru_sequence if hidden <= SEQ_MAX_H else lib.e2e_gru_sequence_wide
+    L.check(fn(L.ptr(gates), int(gates.stride(0)), L.ptr(out), int(out.stride(0)),
+               L.ptr(frame_off), L.ptr(lens), L.ptr(group_first), L.ptr(group_rows),
+               int(lens.numel()), int(hidden), int(group_first.numel()), len(dirs),
+               L.ptr(fw[0]), L.ptr(fw[1]), int(fw[2]), int(fw[3]),
+               L.ptr(bw[0]), L.ptr(bw[1]), int(bw[2]), int(bw[3]), _stream()))
 
 
 def packed_subsample_ln(x, in_off, out_off, out_len, n_out, stride=1, g=1, weight=None, bias=None, eps=1e-5):

@@ -55,13 +55,35 @@ def write_results(results, tokenizer, best_path, beam_path=None):
                 fbeam.close()
 
 
+def encoder_width(encoder):
+    """The widest recurrence output of an encoder's layers (2H for a bidirectional layer of H units), 0 without any."""
+    import torch
+    return max([l.hidden_size * (2 if l.bidirectional else 1) for l in encoder.modules()
+                if isinstance(l, (torch.nn.LSTM, torch.nn.GRU))] or [0])
+
+
+def decode_bytes_fn(decoder, feat_dim):
+    """``bytes_fn(n_utts, l_max)`` that decode_dataset sizes its batches by: shard.estimate_decode_bytes with the
+    decoder's settings.  An encoder wider than the estimate's default 640 (two directions of 320 units) passes its own
+    width, which the encoder output and the packed first layer's gates scale with; narrower ones keep the default."""
+    import functools
+    from . import shard
+    enc = decoder.asr.encoder
+    width = encoder_width(enc)
+    return functools.partial(shard.estimate_decode_bytes, vocab=decoder.asr.vocab_size, beam=decoder.beam_size,
+                             n_cand=decoder.ctc_beam_size if decoder.apply_ctc else 0, feat_dim=feat_dim,
+                             num_head=decoder.asr.attention.num_head, v_proj=bool(decoder.asr.attention.v_proj),
+                             time_reduction=getattr(enc, "sample_rate", 4),
+                             front_reduction=4 if getattr(enc, "vgg", 1) else 1,
+                             **({"enc_dim": width} if width > 640 else {}))
+
+
 def decode_dataset(decoder, samples, device, max_utts=4096, max_padded_frames=0, max_bytes=None):
     """samples: sequence of (name, feat [L,D] float tensor, truth ids).  Returns the reference's
     result tuples (name, [hyp.outIndex ...], truth) in the order of ``samples``
     (bin/test_asr.py:138-139,159-173), decoding many utterances per ``decode_batch`` call.
     Batches are closed before their estimated footprint (shard.estimate_decode_bytes) exceeds ``max_bytes``
     (default: 80 % of the device's free memory), which is what splits a subword-vocabulary set."""
-    import functools
     import torch
     from . import shard
     lengths = np.array([int(s[1].shape[0]) for s in samples], dtype=np.int64)
@@ -69,11 +91,7 @@ def decode_dataset(decoder, samples, device, max_utts=4096, max_padded_frames=0,
     if max_bytes is None and torch.device(device).type == "cuda":
         max_bytes = int(0.8 * torch.cuda.mem_get_info(device)[0])
     feat_dim = int(samples[0][1].shape[1]) if len(samples) else 160
-    bytes_fn = functools.partial(shard.estimate_decode_bytes, vocab=decoder.asr.vocab_size, beam=decoder.beam_size,
-                                 n_cand=decoder.ctc_beam_size if decoder.apply_ctc else 0, feat_dim=feat_dim,
-                                 num_head=decoder.asr.attention.num_head, v_proj=bool(decoder.asr.attention.v_proj),
-                                 time_reduction=getattr(decoder.asr.encoder, "sample_rate", 4),
-                                 front_reduction=4 if getattr(decoder.asr.encoder, "vgg", 1) else 1)
+    bytes_fn = decode_bytes_fn(decoder, feat_dim)
     for batch in shard.make_batches(np.arange(len(samples)), lengths, max_utts, max_padded_frames, max_bytes, bytes_fn):
         l_max = int(lengths[batch].max())
         feats = torch.zeros(len(batch), l_max, samples[batch[0]][1].shape[1])

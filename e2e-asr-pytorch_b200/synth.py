@@ -36,6 +36,15 @@ TINY_ASR_CFG = {
                   "loc_kernel_size": 10, "loc_kernel_num": 4},
     "decoder": {"module": "LSTM", "dim": 20, "layer": 1, "dropout": 0},
 }
+# The bench model at the standard LAS listener width: four BLSTM layers of 512 units per direction (packed recurrence in
+# the thread-block cluster form, csrc/lstm_seq.cu) and a 512-wide speller.
+WIDE_ASR_CFG = copy.deepcopy(ASR_MODEL_CFG)
+WIDE_ASR_CFG["encoder"]["dim"] = [512, 512, 512, 512]
+WIDE_ASR_CFG["decoder"]["dim"] = 512
+# TINY_ASR_CFG's topology with 512-wide encoder layers and speller, for oracle tests of the wide recurrence.
+TINY_WIDE_ASR_CFG = copy.deepcopy(TINY_ASR_CFG)
+TINY_WIDE_ASR_CFG["encoder"]["dim"] = [512, 512]
+TINY_WIDE_ASR_CFG["decoder"]["dim"] = 512
 TINY_LM_CFG = {"emb_tying": True, "emb_dim": 32, "module": "LSTM", "dim": 32, "n_layers": 2, "dropout": 0.5}
 
 

@@ -391,6 +391,24 @@ int e2e_gru_sequence(const float *gates, long long gates_pitch, float *out, long
                      const float *bias_bw, const float *w_t_bw, int gate_off_bw, int out_off_bw,
                      void *stream);
 
+/* e2e_lstm_sequence / e2e_gru_sequence for wider layers: the same arguments, formulas and results (bit for bit where
+ * both accept H), for H a multiple of 128 up to 1024.  Each (utterance group x direction) runs on a thread-block
+ * cluster of CL CTAs, CL the smallest power of two >= 2 with H / CL <= 384; each CTA owns H / CL units and keeps the
+ * whole previous state [2][H][16] fp32 in shared memory (up to 128 KB).  Other H return E2E_ERR_UNSUPPORTED, and so
+ * does a device on which such a cluster does not fit. */
+int e2e_lstm_sequence_wide(const float *gates, long long gates_pitch, float *out, long long out_pitch,
+                           const int *frame_off, const int *lens, const int *group_first, const int *group_rows,
+                           int N, int H, int n_groups, int n_dirs,
+                           const float *bias_fw, const float *w_t_fw, int gate_off_fw, int out_off_fw,
+                           const float *bias_bw, const float *w_t_bw, int gate_off_bw, int out_off_bw,
+                           void *stream);
+int e2e_gru_sequence_wide(const float *gates, long long gates_pitch, float *out, long long out_pitch,
+                          const int *frame_off, const int *lens, const int *group_first, const int *group_rows,
+                          int N, int H, int n_groups, int n_dirs,
+                          const float *bias_fw, const float *w_t_fw, int gate_off_fw, int out_off_fw,
+                          const float *bias_bw, const float *w_t_bw, int gate_off_bw, int out_off_bw,
+                          void *stream);
+
 /* What RNNLayer does to a layer's output between the recurrence and the projection (src/module.py:1003-1081:
  * LayerNorm over the full output row, then sub-sampling by 'drop' or 'concat'), on packed utterances (csrc/encoder_post.cu):
  *   out[out_off[n] + j][s*W : (s+1)*W] = LN(in[in_off[n] + j*stride + s])      for every n < N, j < out_len[n], s < g
