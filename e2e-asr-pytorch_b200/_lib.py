@@ -60,6 +60,18 @@ SIGNATURES = {
                                        c_void_p, c_void_p, c_void_p,
                                        c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                        c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "e2e_beam_combine_prune_wide": (c_int, [c_void_p, c_int, c_void_p,
+                                            c_void_p, c_int,
+                                            c_void_p, c_void_p,
+                                            c_int, c_int, c_int, c_int, c_int,
+                                            c_void_p, c_void_p,
+                                            c_float, c_float, c_float, c_int,
+                                            c_void_p, c_void_p, c_void_p, c_void_p,
+                                            c_void_p, c_void_p, c_void_p,
+                                            c_void_p,
+                                            c_void_p, c_void_p, c_void_p,
+                                            c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                            c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "e2e_attention_loc_full": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                        c_float, c_float, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                                        c_void_p, c_void_p, c_void_p]),

@@ -15,9 +15,10 @@ LIB_DIR = os.path.join(_HERE, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libe2e_asr_b200.so")
 TC_LIB_PATH = os.path.join(LIB_DIR, "libe2e_asr_b200_tc.so")
 SOURCES = ["abi.cu", "ctc_posterior.cu", "prefix_score.cu", "prefix_lazy.cu", "beam_step.cu", "attention_full.cu", "lstm_step.cu", "conv_split.cu",
-           "conv_igemm_host.cu", "lstm_seq.cu", "encoder_post.cu"]
+           "conv_igemm_host.cu", "lstm_seq.cu", "encoder_post.cu",
+           "beam_wide.cu"]
 TC_SOURCES = ["conv_igemm.cu"]
-HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "conv_igemm.cuh"), os.path.join(CSRC, "softplus_lut.inc"), os.path.join(CSRC, "softplus_poly.inc"), os.path.join(_HERE, "..", "include", "e2e_asr_b200.h")]
+HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "beam_select.cuh"), os.path.join(CSRC, "conv_igemm.cuh"), os.path.join(CSRC, "softplus_lut.inc"), os.path.join(CSRC, "softplus_poly.inc"), os.path.join(_HERE, "..", "include", "e2e_asr_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "--expt-extended-lambda", "-Xcompiler", "-fPIC", "-shared"]
 

@@ -432,13 +432,26 @@ static LazyKernel pick_math(int math)
     return prefix_lazy_kernel<kGather, kMathLut, kFixed, kT, kBig>;
 }
 
+constexpr size_t kLazySmemCap = 200 * 1024;
+
+// The frame tile of a launch: 16-frame tiles for machine-filling launches (more CTAs per SM), 32-frame tiles for the tail
+// (fewer barriers per chain) unless their shared memory exceeds the cap (the column-gather form at beams 18-23 and wider
+// rows of candidates); 0 when not even the 16-frame tile fits.
+static int lazy_tile(bool gather, int math, int threads, int Vp, int B, bool machine_filling)
+{
+    if (!machine_filling && lazy_smem_layout(gather, math, threads, Vp, B, 32).total <= kLazySmemCap) return 32;
+    return lazy_smem_layout(gather, math, threads, Vp, B, 16).total <= kLazySmemCap ? 16 : 0;
+}
 }  // namespace e2e
 
 extern "C" int e2e_ctc_prefix_step_supported(int Vp, int B, int C)
 {
+    using namespace e2e;
     if (B <= 0 || C <= 0 || Vp <= 0) return 0;
     const int SW = (B + 7) / 8, PW = (B * C + 31) / 32;
-    return (2 * SW + PW) <= 32 ? 1 : 0;
+    if (2 * SW + PW > 32) return 0;
+    // the table form of the log-add-exp needs the most shared memory: what fits with it fits with every math
+    return lazy_tile(Vp > kLazyMaxRowFloats, kMathLut, (2 * SW + PW) * 32, Vp, B, true) > 0 ? 1 : 0;
 }
 
 extern "C" int e2e_ctc_prefix_step(const float *x, int Tmax, int U, int Vp, int V, const int *enc_len,
@@ -481,13 +494,13 @@ extern "C" int e2e_ctc_prefix_step(const float *x, int Tmax, int U, int Vp, int 
         return e ? atoi(e) : 200;        // measured (profiles/r02_i_prefix_micro_estrin.jsonl): -10 % at 64 utterances, +6 % at 600
     }();
     const int math = (flags & E2E_PREFIX_POLY_MATH) ? (((flags & E2E_PREFIX_POLY_ESTRIN) || n_run < estrin_below) ? kMathPolyEstrin : kMathPoly) : kMathLut;
-    // 16-frame tiles for machine-filling launches (more CTAs per SM), 32-frame tiles for the tail (fewer barriers per chain)
     static const int small_from = []() {
         const char *e = getenv("E2E_LAZY_SMALL_TILE_FROM");          // tuning knob: utterances from which the 16-frame tile is used
         return e ? atoi(e) : 1500;       // measured: 16-frame tiles win from ~1500 utterances up, 32-frame tiles below (profiles/r02_e_prefix_micro_tiles.jsonl)
     }();
     // (64-frame tiles were measured for the deep tail — profiles/r02_o_prefix_micro_tiles64.jsonl: 1-4 % slower than 32; not built)
-    const int tile = n_run >= small_from ? 16 : 32;
+    const int tile = lazy_tile(gather, math, threads, Vp, B, n_run >= small_from);
+    if (tile == 0) return set_error(E2E_ERR_UNSUPPORTED, "e2e_ctc_prefix_step: B=%d, Vp=%d needs more shared memory than a CTA has", B, Vp);
     LazyKernel kern;
     if (fixed) kern = tile == 16 ? pick_math<false, true, 16, false>(math) : pick_math<false, true, 32, false>(math);
     else if (gather) kern = tile == 16 ? (big ? pick_math<true, false, 16, true>(math) : pick_math<true, false, 16, false>(math))
@@ -502,7 +515,6 @@ extern "C" int e2e_ctc_prefix_step(const float *x, int Tmax, int U, int Vp, int 
         if (rc != E2E_OK) return rc;
     }
     if (L.total > 48 * 1024) {
-        if (L.total > 200 * 1024) return set_error(E2E_ERR_UNSUPPORTED, "e2e_ctc_prefix_step: %zu bytes of shared memory needed", L.total);
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total);
         if (e != cudaSuccess) return set_error(E2E_ERR_LAUNCH, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     }

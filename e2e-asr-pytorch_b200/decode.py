@@ -101,8 +101,8 @@ class BeamDecoder(nn.Module):
         self.max_len_ratio = max_len_ratio
         self.asr = asr
         assert self.asr.enable_att                                     # decode.py:27
-        if not 1 <= beam_size <= 32:
-            raise ValueError("beam_size must be in 1..32 (one warp per hypothesis, <=32 warps per CTA)")
+        if not 1 <= beam_size <= ops.BEAM_MAX:
+            raise ValueError("beam_size must be in 1..%d" % ops.BEAM_MAX)
 
         self.apply_ctc = ctc_weight > 0
         if self.apply_ctc:

@@ -183,12 +183,21 @@ class BeamBuffers:
         self.psi = z(u * b, max(1, n_cand), dt=F32)
 
 
+# Beam sizes: e2e_beam_combine_prune gives every parent its own warp up to BEAM_NARROW_MAX; e2e_beam_combine_prune_wide
+# takes any beam up to BEAM_MAX (the same bits at the narrow sizes).
+BEAM_NARROW_MAX = 32
+BEAM_MAX = 64
+
+
 def beam_combine_prune(buf, att_logits, lm_logits, vocab, step, ctc_weight, lm_weight, eos_threshold=1.5, n_run=0):
-    """One decode step of score combine + eos threshold + top-k + prune for all utterances."""
+    """One decode step of score combine + eos threshold + top-k + prune for all utterances (see e2e_beam_combine_prune;
+    e2e_beam_combine_prune_wide above BEAM_NARROW_MAX hypotheses)."""
     _chk(att_logits, F32, "att_logits")
     _chk(lm_logits, F32, "lm_logits")
     flags = (L.BEAM_USE_CTC if ctc_weight > 0 else 0) | (L.BEAM_USE_LM if lm_logits is not None else 0)
-    L.check(L.load().e2e_beam_combine_prune(
+    lib = L.load()
+    fn = lib.e2e_beam_combine_prune if buf.B <= BEAM_NARROW_MAX else lib.e2e_beam_combine_prune_wide
+    L.check(fn(
         L.ptr(att_logits), int(att_logits.stride(0)), L.ptr(buf.att_stats),
         L.ptr(lm_logits), int(lm_logits.stride(0)) if lm_logits is not None else 0,
         L.ptr(buf.cand), L.ptr(buf.psi),

@@ -398,6 +398,17 @@ class EmbFusion:
         return F.linear(x, self.table)
 
 
+ATT_MAX_SLOTS = 32      # beam slots per utterance the fused attention kernels take (kAfMaxB, csrc/attention_full.cu)
+
+
+def attention_groups(beam):
+    """The beam slots [lo, hi) of each fused attention call: one group up to ATT_MAX_SLOTS, else the fewest groups of
+    near-equal size (beam 40: 20 + 20, beam 64: 32 + 32)."""
+    n = -(-beam // ATT_MAX_SLOTS)
+    size = -(-beam // n)
+    return [(lo, min(beam, lo + size)) for lo in range(0, beam, size)]
+
+
 class BatchedStepper:
     def __init__(self, asr, lm=None, split_gemm=False, fused_attention=False, lm_split="bf16x3", vgg_split="bf16x3", step_graphs=False,
                  vgg_conv="igemm", emb=None):
@@ -505,6 +516,7 @@ class BatchedStepper:
         att = self.asr.attention
         u, t, _ = enc.shape
         self.U, self.B, self.T, self.N = u, beam, t, u * beam
+        self._groups = attention_groups(beam)
         dev = enc.device
         if self.H == 1:
             self.fused_step = self.fused_attention
@@ -547,7 +559,8 @@ class BatchedStepper:
         if self.fused_attention and enc.is_cuda:
             from . import ops
             k_filt, _, width = self._w_conv.shape
-            self.fused_step = ops.attention_loc_heads_supported(beam, h, key.shape[3], k_filt, width)
+            widest = max(hi - lo for lo, hi in self._groups)
+            self.fused_step = ops.attention_loc_heads_supported(widest, h, key.shape[3], k_filt, width)
         value = torch.tanh(att.proj_v(enc)) if att.v_proj else enc               # [U,T,H*E] or [U,T,E]
         if self.fused_step:
             self.key_t, self.key = key.permute(0, 2, 3, 1).contiguous(), None    # [U,H,A,T] channel-major per head
@@ -566,9 +579,7 @@ class BatchedStepper:
         elif self.mode == "loc" and self.fused_attention:
             from . import ops
             # conv + energies + masked softmax + context in one kernel (csrc/attention_full.cu)
-            attn, context = ops.attention_loc_full(self.key_t, self.value, query.contiguous(), self.prev_att, self._enc_len32,
-                                                   self._w_conv, self._w_proj, self._w_energy, self._b_energy,
-                                                   self.temperature, b, n_run=k)
+            attn, context = self._fused_attention(ops.attention_loc_full, query, k)
         else:
             if self.mode == "loc":
                 lay = att.att_layer
@@ -583,6 +594,31 @@ class BatchedStepper:
             context = torch.bmm(attn, self.value[:k]).view(n, -1)                      # module.py:1114
         return attn, context
 
+    def _fused_attention(self, fn, query, k, *per_head_values):
+        """ops.attention_loc_full / attention_loc_heads for the first k utterances, once per group of beam slots
+        (self._groups).  The kernels take at most ATT_MAX_SLOTS slots per utterance and their results do not depend on how
+        slots are grouped, so a wider beam runs group by group: each group's query and previous-alignment rows are made
+        contiguous, and its alignments and contexts are scattered back into beam order."""
+        b = self.B
+        args = (self.key_t, self.value)
+        tail = (self._enc_len32, self._w_conv, self._w_proj, self._w_energy, self._b_energy, self.temperature)
+        if len(self._groups) == 1:
+            return fn(*args, query.contiguous(), self.prev_att, *tail, b, *per_head_values, n_run=k)
+        n = k * b
+        q = query.view(k, b, -1)
+        prev = self.prev_att[:n].view(k, b, *self.prev_att.shape[1:])
+        attn = ctx = None
+        for lo, hi in self._groups:
+            g = hi - lo
+            a, c = fn(*args, q[:, lo:hi].reshape(k * g, -1), prev[:, lo:hi].reshape(k * g, *prev.shape[2:]), *tail, g,
+                      *per_head_values, n_run=k)
+            if attn is None:
+                attn = a.new_empty((k, b) + tuple(a.shape[1:]))
+                ctx = c.new_empty((k, b) + tuple(c.shape[1:]))
+            attn[:, lo:hi] = a.view(k, g, *a.shape[1:])
+            ctx[:, lo:hi] = c.view(k, g, *c.shape[1:])
+        return attn.view(n, *attn.shape[2:]), ctx.view(n, -1)
+
     def _attend_heads(self, query, k):
         """One attention step of H > 1 heads for the first k utterances: (alignments [k*B,H,T], merge_head(context))."""
         att, h = self.asr.attention, self.H
@@ -591,9 +627,7 @@ class BatchedStepper:
         if self.fused_step:
             from . import ops
             # conv over the H alignments + energies + masked softmax + per-head contexts in one kernel (csrc/attention_full.cu)
-            attn, ctx = ops.attention_loc_heads(self.key_t, self.value, query.contiguous(), self.prev_att, self._enc_len32,
-                                                self._w_conv, self._w_proj, self._w_energy, self._b_energy, self.temperature, b,
-                                                att.v_proj, n_run=k)
+            attn, ctx = self._fused_attention(ops.attention_loc_heads, query, k, att.v_proj)
         else:
             q = query.view(k, b, h, -1)
             if self.mode == "loc":

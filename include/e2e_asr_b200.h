@@ -130,7 +130,8 @@ int e2e_ctc_prefix_score(const float *x, int Tmax, int U, int Vp, int V, const i
  *   r_out       [U][Tmax][B][2]  out: states of the live hypotheses, rows t >= max(1, len-1) - 1 (earlier rows are
  *               log-zero by construction, never read back, and not written)
  * flags: 0 or E2E_PREFIX_POLY_MATH (| E2E_PREFIX_POLY_ESTRIN).  Needs ceil(B/8) + ceil(B*C/32) <= 32 warps per
- * utterance (e2e_ctc_prefix_step_supported). */
+ * utterance and a frame tile whose shared memory fits (e2e_ctc_prefix_step_supported; the launch takes the 16-frame
+ * tile where the 32-frame one does not fit, so whatever is supported launches at every n_run). */
 int e2e_ctc_prefix_step_supported(int Vp, int B, int C);
 int e2e_ctc_prefix_step(const float *x, int Tmax, int U, int Vp, int V, const int *enc_len,
                         const float *r_prev, int lanes_prev,
@@ -199,6 +200,24 @@ int e2e_beam_combine_prune(const float *att_logits, int ld_att, const float *att
                            int *fin_count, int *fin_step, int *fin_parent, float *fin_sum, float *fin_score,
                            int fin_cap, int *status, int n_run,
                            long long *parent_row, long long *last_tok64, int *parent_tok, void *stream);
+
+/* (3b) for beams up to 64: the arguments, checks and results of e2e_beam_combine_prune, with B in 1..64 (at B <= 32 the
+ * same bits).  One CTA per utterance whose warps loop over the parents, and a pooled prune that ranks each child by binary
+ * search in the other parents' lists.  E2E_ERR_UNSUPPORTED when the shape needs more shared memory than one CTA has
+ * (a candidate count C in the thousands). */
+int e2e_beam_combine_prune_wide(const float *att_logits, int ld_att, const float *att_stats,
+                                const float *lm_logits, int ld_lm,
+                                const int *cand, const float *psi,
+                                int U, int B, int V, int C, int step,
+                                const int *min_len, const int *max_len,
+                                float ctc_weight, float lm_weight, float eos_threshold, int flags,
+                                int *n_live, int *n_active, int *last_tok, int *prefix_len,
+                                float *score_sum, float *ctc_prob, int *prev_lane,
+                                int *parent_slot,
+                                int *hist_tok, int *hist_parent, float *hist_score,
+                                int *fin_count, int *fin_step, int *fin_parent, float *fin_sum, float *fin_score,
+                                int fin_cap, int *status, int n_run,
+                                long long *parent_row, long long *last_tok64, int *parent_tok, void *stream);
 
 /* Final N-best selection + back-tracking.  Replaces src/decode.py:180-183 and
  * Hypothesis.outIndex (src/decode.py:279-281): closed hypotheses followed by the last
